@@ -2,7 +2,7 @@
 """Benchmark of the GLAMR global-optimisation hot path (BASELINE.json metric: global-opt iterations/sec over
 frames x persons), one process per GPU.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--extras all|none|a,b,..]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--extras all|none|a,b,..] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
 
 One "step" = one optimiser iteration of GlobalReconOptimizer.optimize_main (trajectory codec + camera + full SMPL
@@ -63,7 +63,14 @@ def parse():
     ap.add_argument('--extras', default='all', help="'all', 'none' or a comma list of " + ','.join(ALL_EXTRAS))
     ap.add_argument('--cpu-sample-iters', type=int, default=20)
     ap.add_argument('--no-cpu-baseline', action='store_true')
-    return ap.parse_args()
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='write what the last timed step computed (optimisation variables and per-frame outputs) as DIR/<name>.npy')
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error('--steps must be at least 1')
+    if a.dump_outputs and a.impl != 'ours':
+        ap.error('--dump-outputs applies to --impl ours')
+    return a
 
 
 def refuse_experiment_switches():
@@ -478,6 +485,38 @@ class StageLoop:
         self.graph, self.step = None, None
 
 
+PER_PERSON_OUTPUTS = ['smpl_orient_world', 'root_trans_world', 'smpl_orient_world_base', 'root_trans_world_base', 'kp_2d_pred',
+                      'smpl_orient_cam_in_world', 'root_trans_cam_in_world', 'joints_world', 'traj_local']
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(model, data, out_dir, rank):
+    """Write what the last timed step computed, as optimize_main hands it back to its caller: the optimisation variables
+    (theta, every variable of the stage packed) and the per-frame outputs of that step's closure, persons concatenated along
+    axis 0.  All float32.  Above DUMP_LIMIT_BYTES each array keeps a fixed seeded sample of its rows, so that two builds run
+    with the same arguments write the same elements.  Collective when frame-persons are sharded over ranks; rank 0 writes."""
+    model._scatter_outputs(data)
+    if rank != 0:
+        return None
+    import torch
+    persons = list(data['person_data'].values())
+    arrays = {'theta': model._theta, 'cam_pose': data['cam_pose'], 'cam_pose_inv': data['cam_pose_inv']}
+    for k in PER_PERSON_OUTPUTS:
+        arrays[k] = torch.cat([d[k] for d in persons])
+    arrays = {k: v.detach().float().cpu().numpy() for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    sampled = total > DUMP_LIMIT_BYTES
+    if sampled:
+        rng = np.random.default_rng(0)
+        for k, a in arrays.items():
+            n = max(1, a.shape[0] * DUMP_LIMIT_BYTES // total)
+            arrays[k] = a[np.sort(rng.choice(a.shape[0], n, replace=False))]
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + '.npy'), a)
+    return {'dir': out_dir, 'arrays': sorted(arrays), 'bytes': sum(a.nbytes for a in arrays.values()), 'sampled_rows': sampled}
+
+
 def measure_fp32_peak(ctx):
     """TFLOP/s of a register-resident FFMA loop on this GPU right now (best of 5 launches of ~1 ms)"""
     from glamr_b200 import lib as L
@@ -680,6 +719,8 @@ def run_ours(args):
     cold_ms, warm_ms = loop.time(K)
     clocks = sampler.stop() if rank == 0 else None
     _dbg('timed loops done')
+    # before lbs_ms below, which runs further iterations of the same model
+    dumped = dump_outputs(model, data, args.dump_outputs, rank) if args.dump_outputs else None
     lbs_ms = loop.lbs_ms(min(K, 50))
     blend_ms = loop.blend_ms()
     lbs_parts = dict(getattr(loop, 'lbs_parts', {}))
@@ -795,6 +836,8 @@ def run_ours(args):
             'roofline': roofline,
             'extras': extras,
         }
+        if dumped is not None:
+            res['outputs_dump'] = dumped
         if parity is not None:
             res['parity'] = parity
             bad = not parity['ok']

@@ -61,7 +61,7 @@ class _BiLSTM(nn.Module):
         self.rnn_b = nn.LSTMCell(din, dout // 2)
 
     def _run(self, cell, x, reverse):
-        h = torch.zeros(x.shape[1], cell.hidden_size)
+        h = torch.zeros(x.shape[1], cell.hidden_size, dtype=x.dtype)
         c = torch.zeros_like(h)
         outs = [None] * x.shape[0]
         for t in (reversed(range(x.shape[0])) if reverse else range(x.shape[0])):
@@ -121,7 +121,8 @@ class MotionInfiller(nn.Module):
     def inference(self, batch):
         """multi-step, sample_num 1 (:618-652): in_body_pose [B,T,69], frame_mask [B,T] (1 = visible),
         optional in_motion_latent [n_windows,128] -> infer_out_body_pose [B,1,T,69]"""
-        pose = batch['in_body_pose'].transpose(0, 1).contiguous().float().clone()        # [T,B,69]
+        dt = self.data_decoder.out_fc.weight.dtype                                       # float32 (reference); float64 in the fixture check
+        pose = batch['in_body_pose'].transpose(0, 1).contiguous().to(dt).clone()         # [T,B,69]
         key_pad_all = ~(batch['frame_mask'] == 1)                                        # True where NOT visible
         T, B = pose.shape[0], pose.shape[1]
         W = PAST + CUR + FUT
@@ -132,11 +133,11 @@ class MotionInfiller(nn.Module):
             win = pose[s:eb]
             kp = key_pad_all[:, s:eb]
             if e > eb:
-                win = torch.cat([win, torch.zeros(e - eb, B, 69)], dim=0)
+                win = torch.cat([win, torch.zeros(e - eb, B, 69, dtype=dt)], dim=0)
                 kp = torch.cat([kp, torch.ones(B, e - eb, dtype=torch.bool)], dim=1)
             kp = kp.clone()
             kp[:, :PAST] = False
-            eps = batch['in_motion_latent'][[i]].float() if 'in_motion_latent' in batch else None
+            eps = batch['in_motion_latent'][[i]].to(dt) if 'in_motion_latent' in batch else None
             out = self.window(win, kp, eps)
             nfr = min(e - FUT, T) - s
             pose[s:s + nfr] = out[:nfr]
@@ -207,7 +208,7 @@ class MotionTrajJoint:
         flat = body.reshape(-1, 69)
         z3 = torch.zeros_like(flat[:, :3])
         joints = self.smpl.get_joints(z3, flat, root_trans=z3)[:, 1:].reshape(B, T, 69).transpose(0, 1).contiguous()
-        eps = batch['in_traj_latent'].float() if 'in_traj_latent' in batch else None
+        eps = batch['in_traj_latent'].to(body.dtype) if 'in_traj_latent' in batch else None
         local, trans, orient = self.traj_predictor.inference(joints, eps)
         data['infer_out_local_traj_tp'] = local.view(T, B, 1, 11)
         data['infer_out_trans'] = trans.transpose(0, 1).unsqueeze(1).contiguous()

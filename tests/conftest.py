@@ -8,24 +8,19 @@ if REPO not in sys.path:
     sys.path.insert(0, REPO)
 
 GOLDEN = os.path.join(REPO, 'tests', 'golden')
-REFERENCE_ROOT = os.environ.get('GLAMR_REFERENCE_ROOT', '/root/reference')
 
 
 def pytest_configure(config):
     config.addinivalue_line('markers', 'gpu: needs a CUDA device (run on the B200 box with -m gpu)')
-    config.addinivalue_line('markers', 'reference: needs /root/reference (build container only)')
 
 
 def pytest_collection_modifyitems(config, items):
-    have_ref = os.path.isdir(os.path.join(REFERENCE_ROOT, 'global_recon'))
     try:
         import torch
         have_gpu = torch.cuda.is_available()
     except Exception:
         have_gpu = False
     for item in items:
-        if 'reference' in item.keywords and not have_ref:
-            item.add_marker(pytest.mark.skip(reason='reference tree not present'))
         if 'gpu' in item.keywords and not have_gpu:
             item.add_marker(pytest.mark.skip(reason='no CUDA device'))
 

@@ -1,7 +1,8 @@
 """Generate the golden fixtures under tests/golden/ by EXECUTING THE UNMODIFIED REFERENCE (/root/reference)
 through the import shims of oracle/refshim (SURVEY.md Appendix C).  Run in the build container only:
 
-    python tests/golden/make_golden.py            # rewrites tests/golden/*.npz
+    python tests/golden/make_golden.py            # rewrites tests/golden/*.npz and configs.json
+    python tests/golden/make_golden.py configs    # only configs.json (the reference's shipped YAML configs)
 
 The reference ships no tests and no golden vectors (SURVEY.md §4), so these outputs of the reference itself are
 what pins the oracle (tests/test_oracle_vs_golden.py) and, through it, the CUDA path.  Inputs are regenerated
@@ -9,6 +10,7 @@ from seeds by glamr_b200.synthetic; only reference OUTPUTS (plus the learned-pri
 are stored, so the fixtures stay small.
 """
 import copy
+import json
 import os
 import sys
 
@@ -282,6 +284,40 @@ def nets_vectors():
     return out
 
 
+def nets_c3_float64_vectors():
+    """The C3-shape run of nets_vectors with the reference networks, its SMPL and the inputs in float64 (default dtype float64
+    while the reference builds and runs, so that the state its modules create is float64 too): per-sequence sums of all 64
+    sequences.  The trajectory is integrated over 120 frames; with the seeded stand-in weights the heading reaches a few
+    hundred radians, where one float32 ulp is 3e-5 rad, so float32 sums differ from host to host (thread count, SIMD width)
+    by more than the 1e-5 the oracle is held to.  In float64 they do not."""
+    from motion_infiller.models.motion_traj_joint_model import MotionTrajJointModel
+    from motion_infiller.utils.config_motion_traj import Config as MTConfig
+    from glamr_b200.synthetic_nets import make_prior_states
+    sys.path.insert(0, os.path.join(REPO, 'tests'))
+    from helpers import c3_prior_inputs
+    batch = {k: v.double() if v.is_floating_point() else v for k, v in c3_prior_inputs().items()}   # drawn in float32, as the tests draw them
+    torch.set_default_dtype(torch.float64)
+    try:
+        mt = MotionTrajJointModel(MTConfig('joint_motion_traj_demo'), torch.device('cpu'), None)
+        st_m, st_t = make_prior_states(1234)
+        for mod, st in [(mt.mfiller, st_m), (mt.traj_predictor, st_t)]:
+            res = mod.load_state_dict({k: torch.tensor(v) for k, v in st.items()}, strict=False)
+            assert not res.unexpected_keys
+        for mod in (mt.mfiller, mt.traj_predictor, mt.smpl):          # buffers loaded from float32 files (the SMPL models)
+            mod.double()
+        res = mt.inference(batch, sample_num=1)
+    finally:
+        torch.set_default_dtype(torch.float32)
+    out = {}
+    for k, bdim in [('infer_out_body_pose', 0), ('infer_out_local_traj_tp', 1), ('infer_out_orient', 0), ('infer_out_trans', 0)]:
+        v = res[k].detach()
+        assert v.dtype == torch.float64, k
+        red = [d for d in range(v.dim()) if d != bdim]
+        out[f'c3_b64_t120/{k}/sum'] = v.sum(dim=red).numpy()
+        out[f'c3_b64_t120/{k}/abs_sum'] = v.abs().sum(dim=red).numpy()
+    return out
+
+
 def globalopt_case(assets, name, cfg_id, P, T, gaps, niters):
     in_dict = make_in_dict(assets, P, T, seed=0, gaps=gaps, seq_name=name)
     model, cfg = ref_env.make_reference_optimizer(cfg_id, niters=niters)
@@ -389,7 +425,28 @@ def evaluator_vectors():
     return out
 
 
+def config_vectors():
+    """the six shipped configs of the reference (global_recon/cfg/<id>.yml) as parsed by yaml.safe_load: the stage / weight
+    tables that glamr_b200.config.builtin_config_dict rebuilds"""
+    import yaml
+    from glamr_b200.config import BUILTIN_IDS
+    out = {}
+    for cfg_id in BUILTIN_IDS:
+        with open(os.path.join(ref_env.REF_ROOT, 'global_recon', 'cfg', cfg_id + '.yml')) as f:
+            d = yaml.safe_load(f)
+        out[cfg_id] = {k: d[k] for k in ['grecon_model_name', 'dataset', 'grecon_model_specs', 'opt_stage_specs']}
+    return out
+
+
+def write_configs():
+    with open(os.path.join(HERE, 'configs.json'), 'w') as f:
+        json.dump(config_vectors(), f, indent=1, sort_keys=True)
+
+
 def main(only=None):
+    if only == 'configs':
+        write_configs()
+        return
     if only == 'evaluator':
         np.savez_compressed(os.path.join(HERE, 'evaluator.npz'), **evaluator_vectors())
         return
@@ -398,6 +455,10 @@ def main(only=None):
         return
     if only == 'nets':
         np.savez_compressed(os.path.join(HERE, 'nets.npz'), **nets_vectors())
+        np.savez_compressed(os.path.join(HERE, 'nets_c3_f64.npz'), **nets_c3_float64_vectors())
+        return
+    if only == 'nets_c3_f64':
+        np.savez_compressed(os.path.join(HERE, 'nets_c3_f64.npz'), **nets_c3_float64_vectors())
         return
     assets = make_smpl_assets(0)
     if only is not None:                       # one global-opt case by name (adding a fixture without touching the others)
@@ -405,10 +466,12 @@ def main(only=None):
         np.savez_compressed(os.path.join(HERE, f'globalopt_{case[0]}.npz'), **globalopt_case(assets, *case))
         print('wrote', case[0])
         return
+    write_configs()
     np.savez_compressed(os.path.join(HERE, 'rotations.npz'), **rotation_vectors())
     np.savez_compressed(os.path.join(HERE, 'traj_codec.npz'), **traj_vectors())
     np.savez_compressed(os.path.join(HERE, 'smpl.npz'), **smpl_vectors(assets))
     np.savez_compressed(os.path.join(HERE, 'nets.npz'), **nets_vectors())
+    np.savez_compressed(os.path.join(HERE, 'nets_c3_f64.npz'), **nets_c3_float64_vectors())
     for case in GLOBALOPT_CASES:
         rec = globalopt_case(assets, *case)
         np.savez_compressed(os.path.join(HERE, f'globalopt_{case[0]}.npz'), **rec)

@@ -1,15 +1,15 @@
 """CPU-only checks: the C-ABI library exports every symbol include/glamr_b200.h declares (no compute calls), struct
 layouts agree with the ctypes mirror, the built-in stage tables equal the reference YAML, the product refuses CPU."""
 import ctypes
+import json
 import numpy as np
 import os
 
 import pytest
 import torch
-import yaml
 
 import __graft_entry__ as ge
-from conftest import REFERENCE_ROOT
+from conftest import GOLDEN
 from glamr_b200 import lib as L
 from glamr_b200.config import BUILTIN_IDS, Config, builtin_config_dict
 
@@ -47,10 +47,11 @@ def test_product_requires_cuda_device():
         L.require_cuda('cpu')
 
 
-@pytest.mark.reference
 @pytest.mark.parametrize('cfg_id', BUILTIN_IDS)
 def test_builtin_configs_equal_reference_yaml(cfg_id):
-    ref = yaml.safe_load(open(os.path.join(REFERENCE_ROOT, 'global_recon', 'cfg', cfg_id + '.yml')))
+    """tests/golden/configs.json: the reference's global_recon/cfg/<cfg_id>.yml as parsed by yaml.safe_load"""
+    with open(os.path.join(GOLDEN, 'configs.json')) as f:
+        ref = json.load(f)[cfg_id]
     mine = builtin_config_dict(cfg_id)
     assert mine['grecon_model_specs'] == ref['grecon_model_specs']
     assert mine['opt_stage_specs'] == ref['opt_stage_specs']

@@ -28,8 +28,12 @@ def test_motion_traj_inference_matches_reference(tag, joint_model):
         np.testing.assert_allclose(out[k].numpy(), g[f'{tag}/{k}'], atol=tol, err_msg=f'{tag} {k}')
 
 
-def test_c3_shape_matches_reference(joint_model):
-    """BASELINE.json configs[2] shape: 64 x 120 with frames 40-69 masked"""
+def test_c3_shape_matches_reference(joint_model, smpl_assets):
+    """BASELINE.json configs[2] shape: 64 x 120 with frames 40-69 masked.  Four whole sequences element-wise in float32; all 64
+    through per-sequence sums, in float64 for every output (tests/golden/nets_c3_f64.npz: the reference run in float64).  The
+    float32 sums of the translation are not compared: it integrates a heading that reaches a few hundred radians over 120
+    frames (seeded stand-in weights), where one float32 ulp is 3e-5 rad, so its float32 sums change with the host's
+    thread count and SIMD width by more than 1e-5."""
     from helpers import C3_ROWS, c3_prior_inputs
     g = load_golden('nets')
     out = joint_model.inference(c3_prior_inputs(), sample_num=1)
@@ -37,4 +41,15 @@ def test_c3_shape_matches_reference(joint_model):
     for k, bdim, tol in [('infer_out_body_pose', 0, 2e-5), ('infer_out_local_traj_tp', 1, 2e-5), ('infer_out_trans', 0, 1e-4), ('infer_out_orient', 0, 1e-4)]:
         np.testing.assert_allclose(out[k].index_select(bdim, sel).numpy(), g[f'c3_b64_t120/{k}'], atol=tol, err_msg=k)
         red = [d for d in range(out[k].dim()) if d != bdim]
-        np.testing.assert_allclose(out[k].double().abs().sum(dim=red).numpy(), g[f'c3_b64_t120/{k}/abs_sum'], rtol=1e-5, err_msg=k)
+        if k != 'infer_out_trans':
+            np.testing.assert_allclose(out[k].double().abs().sum(dim=red).numpy(), g[f'c3_b64_t120/{k}/abs_sum'], rtol=1e-5, err_msg=k)
+    st_m, st_t = make_prior_states(1234)
+    model64 = MotionTrajJoint(st_m, st_t, OracleSMPL(smpl_assets, dtype=torch.float64))
+    model64.mfiller.double()
+    model64.traj_predictor.double()
+    g64 = load_golden('nets_c3_f64')
+    out = model64.inference({k: v.double() if v.is_floating_point() else v for k, v in c3_prior_inputs().items()}, sample_num=1)
+    for k, bdim in [('infer_out_body_pose', 0), ('infer_out_local_traj_tp', 1), ('infer_out_trans', 0), ('infer_out_orient', 0)]:
+        assert out[k].dtype == torch.float64, k
+        red = [d for d in range(out[k].dim()) if d != bdim]
+        np.testing.assert_allclose(out[k].abs().sum(dim=red).numpy(), g64[f'c3_b64_t120/{k}/abs_sum'], rtol=1e-5, err_msg=k + ' (float64)')
