@@ -28,12 +28,8 @@
 #endif
 
 // Which implementation runs when the environment does not say otherwise.  A path becomes the default only after its parity
-// tests passed on a B200 (GLAMR_ITER_PATH=fused|legacy, GLAMR_LBS_PATH=tc|simt select explicitly for A/B runs).
-#define GLAMR_DEFAULT_ITER_FUSED 0
+// tests passed on a B200 (GLAMR_LBS_PATH=tc|tcblend|simt selects explicitly for A/B runs).
 #define GLAMR_DEFAULT_LBS_TC 2        /* 2 = tensor-core blend + tensor-core skinning (verified on B200: all GPU tests green, memcheck clean), 1 = tensor-core blend + SIMT skinning, 0 = FP32 SIMT kernel */
-#define GLAMR_DEFAULT_BLEND_EARLY 0    /* 1: pipelined blend at the top of the evaluation into a second v_posed buffer -- measured slower (it takes the SMs the skinning needs: 98.8 vs 88.0 us at 1 x 300), kept selectable (GLAMR_BLEND_EARLY=1) */
-#define GLAMR_DEFAULT_BLEND_SPLIT 0    /* percent of the pipelined blend launched at the top of the evaluation (GLAMR_BLEND_SPLIT) */
-#define GLAMR_DEFAULT_SMEM_CARVEOUT 3   /* bit mask, see smem_carveout_mask() in smpl_kernels.cu: measured 193.0 -> 157.4 us per iteration at 4 x 300, neutral at 1 x 300 */
 #define GLAMR_DEFAULT_NET_WIMG 0       /* prior-network GEMMs: weight operand as a pre-split image fetched by bulk TMA (GLAMR_NET_WIMG=1) */
 
 namespace glamr {
@@ -108,12 +104,6 @@ __device__ __forceinline__ void tma_bulk_g2s(void* smem_dst, const void* gsrc, u
                : "memory");
 }
 
-// ---- programmatic dependent launch (PDL): every kernel of the optimiser iteration is launched with the
-// programmatic-stream-serialization attribute, lets the next kernel be scheduled early (launch_dependents) and
-// waits for the previous grid's results (wait) only where it first touches them.
-__device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
-__device__ __forceinline__ void pdl_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
-
 // ---- tcgen05 (UMMA) helpers: shared-memory descriptor of a K-major, un-swizzled operand tile and one kind::tf32 MMA ----
 // rows = rows of the operand tile (128 for X, NT for W): fixes the leading byte offset between 16-byte K groups
 __device__ __forceinline__ uint64_t umma_desc_kmajor_noswizzle(const void* smem_ptr, int rows) {
@@ -153,34 +143,5 @@ __device__ __forceinline__ double warp_sum(double v) {
   for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
   return v;
 }
-
-#if defined(__CUDACC__)
-// GLAMR_PDL = bit mask of the kernels launched with the attribute (A/B runs): 1 traj/cam forward, 2 pose_prep, 4 lbs,
-// 8 residuals, 16 traj/cam backward (+ mode-3 camera kernels), 32 apply
-constexpr int kPdlDefaultMask = 0;
-inline bool pdl_enabled(int bit) {
-  static int mask = -1;
-  if (mask < 0) {
-    const char* e = getenv("GLAMR_PDL");
-    mask = e ? atoi(e) : kPdlDefaultMask;
-  }
-  return (mask & bit) != 0;
-}
-// kernel<<<grid, block, smem, s>>>(args...) with the PDL attribute (GLAMR_PDL=0 falls back to a plain launch for A/B runs)
-template <typename... KArgs, typename... Args>
-inline cudaError_t launch_pdl(int bit, void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t s, Args... args) {
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = grid;
-  cfg.blockDim = block;
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = s;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = pdl_enabled(bit) ? 1 : 0;
-  return cudaLaunchKernelEx(&cfg, kernel, KArgs(args)...);
-}
-#endif
 
 }  // namespace glamr

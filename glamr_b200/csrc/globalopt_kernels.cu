@@ -53,8 +53,6 @@ __device__ bool grid_last_block(unsigned int* ticket) {
 // blocks [0,P): trajectory codec of one person; blocks [P, P+cam_blocks): camera of 256 frames each (modes 0-2)
 __global__ void __launch_bounds__(kScanThreads) traj_cam_forward_kernel(OptCtx c, int with_cam) {
   __shared__ float sm[kScanThreads / 32 + 1];
-  pdl_launch_dependents();
-  pdl_wait();
   // [grad | term sums] of this iteration start from zero (the previous iteration's apply has consumed them)
   for (int i = blockIdx.x * kScanThreads + threadIdx.x; i < c.pb.n_params + GLAMR_NUM_TERMS; i += gridDim.x * kScanThreads) c.sc.grad[i] = 0.0f;
   if ((int)blockIdx.x >= c.pb.P) {
@@ -79,8 +77,6 @@ __global__ void __launch_bounds__(kScanThreads) traj_cam_forward_kernel(OptCtx c
 }
 
 __global__ void __launch_bounds__(kFrameThreads) cam_forward_kernel(OptCtx c) {
-  pdl_launch_dependents();
-  pdl_wait();
   const int t = blockIdx.x * blockDim.x + threadIdx.x;
   if (t < c.pb.T) cam_forward(c, t);
 }
@@ -89,8 +85,6 @@ __global__ void __launch_bounds__(kFrameThreads) cam_forward_kernel(OptCtx c) {
 // reprojection terms, warp-shuffle sums, then lane 0 finishes the per-frame terms.  4 frame-persons per CTA.
 __global__ void __launch_bounds__(kFrameThreads) frame_residuals_kernel(OptCtx c, SmplDev m, SmplWorkspace wo, int n_begin, double* partial) {
   __shared__ double sm[(kFrameThreads / 32) * GLAMR_NUM_TERMS];
-  pdl_launch_dependents();
-  pdl_wait();
   const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
   const int n = blockIdx.x * (kFrameThreads / 32) + wid;
   const int N = c.pb.P * c.pb.T, J = c.pb.J;
@@ -157,8 +151,6 @@ extern "C" int glamr_exp_frame_stamps(long long* out32) {     // experiment buil
 
 __global__ void __launch_bounds__(kFrameThreads) camera_backward_kernel(OptCtx c, double* partial) {
   __shared__ double sm[(kFrameThreads / 32) * GLAMR_NUM_TERMS];
-  pdl_launch_dependents();
-  pdl_wait();
   const int t = blockIdx.x * blockDim.x + threadIdx.x;
   TermAcc acc;
   acc.clear();
@@ -167,8 +159,6 @@ __global__ void __launch_bounds__(kFrameThreads) camera_backward_kernel(OptCtx c
 }
 
 __global__ void __launch_bounds__(kFrameThreads) camera_scatter_kernel(OptCtx c) {
-  pdl_launch_dependents();
-  pdl_wait();
   const int s = blockIdx.x * blockDim.x + threadIdx.x;
   if (s < c.pb.T) camera_scatter_to_persons(c, s);
 }
@@ -250,8 +240,6 @@ __global__ void __launch_bounds__(kScanThreads) traj_cam_backward_kernel(OptCtx 
                                                                          int n_slots, float* reduce_buf, unsigned int* ticket, PeerCtx pc) {
   __shared__ float sm[kScanThreads / 32 + 1];
   __shared__ double smd[(kScanThreads / 32) * GLAMR_NUM_TERMS];
-  pdl_launch_dependents();
-  pdl_wait();
   TermAcc acc;
   acc.clear();
   if ((int)blockIdx.x >= c.pb.P) {
@@ -302,22 +290,6 @@ struct AdamState {
   double* beta_pow;   // [0] beta1^t, [1] beta2^t, [2] step count (as a double)
 };
 
-// torch.optim.Adam on theta[lo, hi) with this iteration's bias corrections (same arithmetic as apply_kernel)
-__device__ __forceinline__ void adam_range(const OptCtx& c, float* __restrict__ theta, const float* __restrict__ grad, const AdamState& ad, int lo, int hi,
-                                           float bc2s, float step_size) {
-  for (int i = lo + threadIdx.x; i < hi; i += blockDim.x) {
-    if (!c.pb.active[i]) continue;
-    const float g = grad[i];
-    float m = ad.m[i], v = ad.v[i];
-    m = m + 0.1f * (g - m);
-    v = v * 0.999f + 0.001f * g * g;
-    const float denom = sqrtf(v) / bc2s + 1e-8f;
-    theta[i] = theta[i] - step_size * (m / denom);
-    ad.m[i] = m;
-    ad.v[i] = v;
-  }
-}
-
 __device__ void write_losses(const OptCtx& c, const float* term_sums /*[NUM_TERMS] un-normalised*/, float* loss_terms) {
   double total = 0.0;
   for (int k = 0; k < GLAMR_NUM_TERMS; ++k) {
@@ -339,8 +311,6 @@ __global__ void __launch_bounds__(32) losses_kernel(OptCtx c, const float* __res
 // pc.world > 1: the gradient is the rank-ordered sum of every GPU's published slot (peer memory), not reduce_buf.
 __global__ void __launch_bounds__(256) apply_kernel(OptCtx c, float* __restrict__ theta, const float* __restrict__ reduce_buf, double lr,
                                                     AdamState ad, float* loss_terms, int hist_stride, unsigned int* ticket, PeerCtx pc) {
-  pdl_launch_dependents();
-  pdl_wait();
   const double b1 = ad.beta_pow[0] * 0.9, b2 = ad.beta_pow[1] * 0.999, step = ad.beta_pow[2];
   const uint32_t epoch = pc.world > 1 ? reinterpret_cast<const uint32_t*>(pc.bufs[pc.rank])[1] + 1u : 0u;
   if (pc.world > 1) {
@@ -386,252 +356,6 @@ __global__ void __launch_bounds__(256) apply_kernel(OptCtx c, float* __restrict_
     if (pc.world > 1) reinterpret_cast<uint32_t*>(pc.bufs[pc.rank])[1] = epoch;
   }
 }
-
-
-
-// ------------------------------------------------------------------------------------------------ fused head of the iteration
-// trajectory codec + camera + SMPL pose preparation in ONE launch.  CTA (p, j) owns the 16 frames [16 j, 16 j + 16) of person p:
-// it recomputes the person's heading / xy prefix sums up to its last frame in SHARED memory (O(T) trivial flops per CTA instead
-// of a grid-wide dependency on one scanning CTA), finishes the world pose of its own frames, and then runs the kinematic chain of
-// those frames with one warp per frame (pose_prep_frame).  Camera modes 0-2: the CTAs of person 0 also evaluate the camera of
-// their frames.  Results are bit-identical to traj_cam_forward_kernel + pose_prep_kernel (same scan tree, same formulas).
-constexpr int kFwdFrames = kScanThreads / 32;
-__global__ void __launch_bounds__(kScanThreads) forward_pose_kernel(OptCtx c, SmplDev m, SmplWorkspace wo, int n_ws_begin, int with_cam,
-                                                                    int chunks_per_person, int lpad) {
-  extern __shared__ float fwd_dyn[];
-  __shared__ float sm[kScanThreads / 32 + 1];
-  __shared__ float s_orient[kFwdFrames][3];
-  pdl_launch_dependents();
-  pdl_wait();
-  const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
-  for (int i = blockIdx.x * kScanThreads + tid; i < c.pb.n_params + GLAMR_NUM_TERMS; i += gridDim.x * kScanThreads) c.sc.grad[i] = 0.0f;
-  const int p = blockIdx.x / chunks_per_person, j = blockIdx.x - p * chunks_per_person;
-  const int T = c.pb.T;
-  const int t0 = j * kFwdFrames, t1 = min(t0 + kFwdFrames, T);
-  const glamr_person_t& ps = c.pb.persons[p];
-  const int len = ps.len, start = ps.start;
-  const int cnt = min(len, t1 - start);               // local frames [0, cnt) feed this chunk's prefix sums (<= 0: chunk precedes the track)
-  float* s_head = fwd_dyn;
-  float* s_x = fwd_dyn + lpad;
-  float* s_y = fwd_dyn + 2 * lpad;
-  for (int i = tid; i < cnt; i += kScanThreads) {
-    float tl[11];
-    s_head[i] = traj_pre_vals(c, p, i, tl);
-    s_x[i] = tl[0];
-    s_y[i] = tl[1];
-  }
-  __syncthreads();
-  if (cnt > 0) block_scan_inplace(s_head, cnt, 1, false, sm);
-  __syncthreads();
-  for (int i = tid; i < cnt; i += kScanThreads) {
-    if (i > 0) {                                       // traj_utils.py:76-77: d_xy of frame i rotated by heading[i-1]
-      const float h = s_head[i - 1];
-      const float ct = cosf(h), st = sinf(h);
-      const float x = s_x[i], y = s_y[i];
-      s_x[i] = x * ct - y * st;
-      s_y[i] = x * st + y * ct;
-    }
-  }
-  __syncthreads();
-  if (cnt > 0) {
-    block_scan_inplace(s_x, cnt, 1, false, sm);
-    block_scan_inplace(s_y, cnt, 1, false, sm);
-  }
-  __syncthreads();
-  if (tid < t1 - t0) {
-    const int t = t0 + tid, i = t - start;
-    const size_t n = (size_t)p * T + t;
-    float tl[11], head = 0.0f, x = 0.0f, y = 0.0f;
-    if (i >= 0 && i < len) {
-      traj_pre_vals(c, p, i, tl);
-      head = s_head[i]; x = s_x[i]; y = s_y[i];
-      c.sc.heading[n] = head;
-      c.sc.xy[2 * n] = x;
-      c.sc.xy[2 * n + 1] = y;
-    } else {
-#pragma unroll
-      for (int k = 0; k < 11; ++k) tl[k] = 0.0f;
-    }
-#pragma unroll
-    for (int k = 0; k < 11; ++k) c.sc.traj_local[n * 11 + k] = tl[k];
-    float ow[3];
-    traj_post_vals(c, p, t, tl, head, x, y, ow);
-    s_orient[tid][0] = ow[0]; s_orient[tid][1] = ow[1]; s_orient[tid][2] = ow[2];
-  }
-  if (with_cam && p == 0 && tid >= 32 && tid < 32 + (t1 - t0)) cam_forward(c, t0 + tid - 32);
-  __syncthreads();
-  if (wid < t1 - t0) {
-    const int n = p * T + t0 + wid;
-    if (n >= c.pb.n_begin && n < c.pb.n_end)
-      pose_prep_frame(m, n - n_ws_begin, s_orient[wid], c.pb.smpl_pose_all + (size_t)n * 69, c.pb.smpl_beta_all + (size_t)n * kNB, wo, lane);
-  }
-}
-
-// ------------------------------------------------------------------------------------------------ fused tail of the iteration
-// residuals + analytic backward (+ Adam on one GPU) in ONE launch (camera modes 0-2):
-//   phase A  every CTA: one warp per frame-person -- joint assembly, projection, reprojection terms, warp-shuffle sums -> kpg[n]
-//   ticket   per person: the CTA that completes the last frame of person p continues with
-//   phase B  thread per frame: frame_rest (camera-frame pose, cam_traj, smoothness, rel_transform, their gradients), then the
-//            reverse trajectory codec of person p (three reverse scans), regularisers, [Adam on person p's block of theta]
-//   ticket   global: the CTA that finishes the last person runs the camera backward for all frames, folds the fp64 term sums
-//            in fixed slot order, [Adam on the camera block, loss history row, step count].
-// Sums never depend on which CTA happens to be last: every slot is produced by a fixed-order tree and folded in slot order.
-struct FusedArgs {
-  KpGrad* kpg;               // [N] per frame-person joint sums of phase A
-  double* partial;           // [P + 1][NUM_TERMS] slot p: person p, slot P: camera
-  unsigned int* person_ticket;   // [P]
-  unsigned int* global_ticket;   // [1]
-  float* reduce_buf;         // [n_params + NUM_TERMS]
-  float* theta;              // written when do_adam
-  AdamState ad;
-  double lr;
-  float* loss_terms;
-  int hist_stride;
-  int do_adam;
-};
-constexpr int kFusedFramesPerCta = kScanThreads / 32;   // 16 warps -> 16 frame-persons in phase A
-
-__global__ void __launch_bounds__(kScanThreads) residuals_backward_kernel(OptCtx c, SmplDev m, SmplWorkspace wo, int n_ws_begin, FusedArgs a) {
-  __shared__ float sm[kScanThreads / 32 + 1];
-  __shared__ double smd[(kScanThreads / 32) * GLAMR_NUM_TERMS];
-  __shared__ int mine[kFusedFramesPerCta];     // persons this CTA has to finish (a 16-frame window touches <= 2 of them when T >= 16)
-  __shared__ int n_mine;
-  __shared__ bool last_cta;
-  pdl_launch_dependents();
-  pdl_wait();
-  const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
-  const int P = c.pb.P, T = c.pb.T, N = P * T, J = c.pb.J;
-  // Adam constants of THIS iteration (beta powers are advanced by the very last CTA after everybody has read them)
-  const double b1 = a.ad.beta_pow[0] * 0.9, b2 = a.ad.beta_pow[1] * 0.999, step = a.ad.beta_pow[2];
-  const float bc2s = (float)sqrt(1.0 - b2);
-  const float step_size = (float)(a.lr / (1.0 - b1));
-
-  // ---- phase A
-  const int n0 = blockIdx.x * kFusedFramesPerCta;
-  {
-    const int n = n0 + wid;
-    if (n < N && n >= c.pb.n_begin && n < c.pb.n_end) {
-      const int p = n / T, t = n - p * T;
-      const int nl = n - n_ws_begin;
-      const float* tw = c.sc.trans_world + (size_t)n * 3;
-      const float sc = c.pb.scale_all ? c.pb.scale_all[n] : 1.0f;
-      float root[3], Rc[9], tc[3], Rs[9];
-      raw_joint(m, wo, nl, m.joint_map[0], root);
-      mat34_R(c.sc.cam + (size_t)t * 12, Rc);
-      tc[0] = c.sc.cam[(size_t)t * 12 + 3]; tc[1] = c.sc.cam[(size_t)t * 12 + 7]; tc[2] = c.sc.cam[(size_t)t * 12 + 11];
-      rodrigues_smplx(c.sc.orient_world + (size_t)n * 3, Rs);
-      KpGrad kg;
-      kg.clear();
-      for (int k = lane; k < J; k += 32) {
-        float v[3], jw[3];
-        raw_joint(m, wo, nl, m.joint_map[k], v);
-        jw[0] = (v[0] - root[0]) * sc + tw[0];
-        jw[1] = (v[1] - root[1]) * sc + tw[1];
-        jw[2] = (v[2] - root[2]) * sc + tw[2];
-        float* o = c.sc.joints_world + ((size_t)n * J + k) * 3;
-        o[0] = jw[0]; o[1] = jw[1]; o[2] = jw[2];
-        kp_joint_terms(c, p, t, k, jw, Rc, tc, Rs, tw, kg);
-      }
-#pragma unroll
-      for (int k = 0; k < 3; ++k) { kg.g_tc[k] = warp_sum(kg.g_tc[k]); kg.g_tw[k] = warp_sum(kg.g_tw[k]); }
-#pragma unroll
-      for (int k = 0; k < 9; ++k) { kg.g_Rc[k] = warp_sum(kg.g_Rc[k]); kg.g_Rs[k] = warp_sum(kg.g_Rs[k]); }
-      kg.kp = warp_sum(kg.kp);
-      kg.dist = warp_sum(kg.dist);
-      if (lane == 0) a.kpg[n] = kg;
-    }
-  }
-  // ---- per-person tickets: count the frames of each person this CTA covered
-  __threadfence();
-  __syncthreads();
-  if (tid == 0) {
-    int cnt = 0;
-    const int n1 = min(n0 + kFusedFramesPerCta, N);
-    for (int p = n0 / T; p < P && p * T < n1; ++p) {
-      const int lo = max(n0, p * T), hi = min(n1, (p + 1) * T);
-      if (hi <= lo) continue;
-      const unsigned int old = atomicAdd(&a.person_ticket[p], (unsigned int)(hi - lo));
-      if (old + (unsigned int)(hi - lo) == (unsigned int)T) {
-        a.person_ticket[p] = 0u;               // ready for the next iteration (nobody else touches it any more)
-        mine[cnt++] = p;
-      }
-    }
-    n_mine = cnt;
-  }
-  __syncthreads();
-  if (n_mine == 0) return;
-  __threadfence();                              // acquire: kpg of the other CTAs
-
-  for (int q = 0; q < n_mine; ++q) {
-    const int p = mine[q];
-    const glamr_person_t& ps = c.pb.persons[p];
-    const int len = ps.len;
-    const size_t nb = (size_t)p * T + ps.start;
-    TermAcc acc;
-    acc.clear();
-    // ---- phase B1: per-frame residuals of person p
-    for (int t = tid; t < T; t += kScanThreads) {
-      const int n = p * T + t;
-      if (n >= c.pb.n_begin && n < c.pb.n_end) {
-        const KpGrad kg = a.kpg[n];
-        frame_rest(c, p, t, kg, acc);
-      } else {
-#pragma unroll
-        for (int k = 0; k < 3; ++k) { c.sc.g_orient[(size_t)n * 3 + k] = 0.0f; c.sc.g_trans[(size_t)n * 3 + k] = 0.0f; }
-#pragma unroll
-        for (int k = 0; k < 12; ++k) c.sc.g_cam[(size_t)n * 12 + k] = 0.0f;
-      }
-    }
-    __syncthreads();
-    // ---- phase B2: reverse trajectory codec
-    for (int t = tid; t < T; t += kScanThreads) traj_back_pre(c, p, t, acc);
-    __syncthreads();
-    block_scan_inplace(c.sc.g_xy + 2 * nb, len, 2, true, sm);
-    block_scan_inplace(c.sc.g_xy + 2 * nb + 1, len, 2, true, sm);
-    __syncthreads();
-    for (int i = tid; i < len; i += kScanThreads) traj_back_mid(c, p, i, acc);
-    __syncthreads();
-    block_scan_inplace(c.sc.g_head + nb, len, 1, true, sm);
-    __syncthreads();
-    for (int i = tid; i < len; i += kScanThreads) traj_back_post(c, p, i, acc);
-    block_reduce_terms(acc, a.partial + (size_t)p * GLAMR_NUM_TERMS, smd);
-    __syncthreads();                            // this CTA's gradient stores are visible to all of its threads
-    if (a.do_adam) {
-      const int lo = ps.off_xy, hi = (p + 1 < P) ? c.pb.persons[p + 1].off_xy : c.pb.n_params;   // person p's contiguous block of theta
-      adam_range(c, a.theta, a.reduce_buf, a.ad, lo, hi, bc2s, step_size);
-    }
-  }
-  // ---- global ticket over the persons
-  __threadfence();
-  __syncthreads();
-  if (tid == 0) {
-    const unsigned int old = atomicAdd(a.global_ticket, (unsigned int)n_mine);
-    last_cta = (old + (unsigned int)n_mine == (unsigned int)P);
-    if (last_cta) *a.global_ticket = 0u;
-  }
-  __syncthreads();
-  if (!last_cta) return;
-  __threadfence();
-  {
-    TermAcc acc;
-    acc.clear();
-    for (int t = tid; t < T; t += kScanThreads) camera_backward(c, t, acc);
-    block_reduce_terms(acc, a.partial + (size_t)P * GLAMR_NUM_TERMS, smd);
-    __syncthreads();
-    reduce_tail(c, a.partial, P + 1, a.reduce_buf, smd);
-    __syncthreads();
-    if (a.do_adam) {
-      adam_range(c, a.theta, a.reduce_buf, a.ad, 0, c.pb.persons[0].off_xy, bc2s, step_size);     // camera block precedes the persons
-      if (tid == 0) {
-        if (a.loss_terms) write_losses(c, a.reduce_buf + c.pb.n_params, a.loss_terms + (a.hist_stride > 0 ? (size_t)step * a.hist_stride : 0));
-        a.ad.beta_pow[0] = b1;
-        a.ad.beta_pow[1] = b2;
-        a.ad.beta_pow[2] = step + 1.0;
-      }
-    }
-  }
-}
-
 }  // namespace glamr
 
 using namespace glamr;
@@ -644,11 +368,7 @@ struct glamr_opt {
   AdamState adam;
   double* partial;
   int n_slots, slots_res, slots_cam, cam_blocks;   // partial-sum slots: residual CTAs | P + cam_blocks (traj/cam kernel) | slots_cam (mode 3)
-  unsigned int* tickets;                           // [0] backward tail, [1] apply, [2] fused global, [4 .. 4+P) fused per person
-  KpGrad* kpg;                                     // [N] phase-A sums of the fused tail kernel
-  int fused;                                       // fused head (trajectory + camera + pose prep) and fused tail (residuals + backward [+ Adam], camera
-                                                   // modes 0-2) kernels; GLAMR_ITER_PATH=legacy selects the one-kernel-per-phase path
-  size_t fwd_smem_set;
+  unsigned int* tickets;                           // [0] backward tail, [1] apply, [3] stand-alone peer all-reduce
   void* arena;
   size_t arena_bytes;
   float gs[GLAMR_NUM_TERMS];
@@ -661,8 +381,6 @@ struct glamr_opt {
   int vpt_ready;
   int join_pending;           // a glamr_opt_backward_for_apply call left the side stream un-joined (the next call on the handle joins)
   int features_early;         // the pipelined blend's feature kernel runs at the top of the evaluation
-  int blend_split;            // percent of the pipelined blend's frame tiles launched at the top of the evaluation (0: none)
-  int blend_early;            // the pipelined blend is launched at the top of the evaluation into the other v_posed buffer
   cudaEvent_t ev[24];         // timing == 2: one event after every launch of glamr_opt_backward / glamr_opt_apply
   int n_ev;
   // glamr_opt_iterate: one captured iteration (backward + apply), valid for the arguments it was captured with
@@ -710,8 +428,7 @@ extern "C" int glamr_opt_create(glamr_opt_t** out, const glamr_smpl_t* smpl, con
   auto take = [&](size_t nfl) { size_t o = floats; floats += (nfl + 63) & ~(size_t)63; return o; };
   const size_t o_partial = take((size_t)st->n_slots * GLAMR_NUM_TERMS * 2);
   const size_t o_beta = take(8);
-  const size_t o_ticket = take(8 + (size_t)pb->P);
-  const size_t o_kpg = take(N * (sizeof(KpGrad) / sizeof(float)));
+  const size_t o_ticket = take(8);
   const size_t o_heading = take(N), o_xy = take(2 * N), o_tl = take(11 * N), o_ob = take(3 * N), o_tb = take(3 * N),
                o_ow = take(3 * N), o_tw = take(3 * N), o_cam = take(12 * T), o_caminv = take(12 * T), o_camd6 = take(6 * T),
                o_jw = take(N * J * 3), o_kp = take(N * J * 2), o_ociw = take(3 * N), o_tciw = take(3 * N), o_go = take(3 * N),
@@ -719,31 +436,16 @@ extern "C" int glamr_opt_create(glamr_opt_t** out, const glamr_smpl_t* smpl, con
                o_m = take(pb->n_params), o_v = take(pb->n_params);
   const size_t o_ws = take(smpl_workspace_floats((int)N, smpl->dev.S));
   {
-    const char* ep = getenv("GLAMR_ITER_PATH");
-    st->fused = ep ? (strcmp(ep, "fused") == 0) : GLAMR_DEFAULT_ITER_FUSED;
-    // GLAMR_BLEND_EARLY=0|1: launch the pipelined blend after the skinning (0) or at the top of the evaluation (1, needs the
-    // second v_posed buffer); the fused iteration advances the step count inside its tail kernel and keeps the single buffer
-    const char* e = getenv("GLAMR_BLEND_EARLY");
-    st->blend_early = (e ? atoi(e) != 0 : GLAMR_DEFAULT_BLEND_EARLY != 0) && !st->fused;
-    // GLAMR_BLEND_SPLIT=<percent>: launch that share of the pipelined blend's 128-frame tiles at the TOP of the evaluation, where the GPU
-    // only runs the latency-bound trajectory / pose kernels, and the rest after the skinning (0: everything after the skinning).
-    // Needs the second v_posed buffer like GLAMR_BLEND_EARLY.
-    const char* sp = getenv("GLAMR_BLEND_SPLIT");
-    st->blend_split = st->fused || st->blend_early ? 0 : (sp ? atoi(sp) : GLAMR_DEFAULT_BLEND_SPLIT);
-    if (st->blend_split < 0 || st->blend_split > 100) st->blend_split = 0;
-    // GLAMR_FEATURES_EARLY=0|1: the feature kernel of the pipelined blend (its A operand; body pose / betas only) runs at the top of the
-    // evaluation on the side stream, so that only the GEMM is left after the skinning
-    // (default: only while this rank's per-frame kernels have fewer CTAs than the GPU has SMs -- measured 102.8 -> 94.8 us per L2-flushed
-    // iteration at 1 x 300, but 154 -> 180 us at 4 x 300, where the GEMM then no longer follows a kernel with its own shared-memory split)
-    const char* fe = getenv("GLAMR_FEATURES_EARLY");
+    // the feature kernel of the pipelined blend (its A operand; body pose / betas only) runs at the top of the evaluation on the side
+    // stream, so that only the GEMM is left after the skinning -- only while this rank's per-frame kernels have fewer CTAs than the GPU
+    // has SMs: measured 102.8 -> 94.8 us per L2-flushed iteration at 1 x 300, but 154 -> 180 us at 4 x 300, where the GEMM then no
+    // longer follows a kernel with its own shared-memory split
     int sms = 148, dev = 0;
     cudaGetDevice(&dev);
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
     const int frame_ctas = (pb->n_end - pb->n_begin + kFrameThreads / 32 - 1) / (kFrameThreads / 32);
-    st->features_early = (fe ? atoi(fe) != 0 : frame_ctas < sms) && !st->fused;
+    st->features_early = frame_ctas < sms;
   }
-  const size_t n128 = (N + kTcM - 1) / kTcM * kTcM;
-  const size_t o_vp2 = (st->blend_early || st->blend_split > 0) ? take((size_t)kTcCols * ((n128 + kSkF - 1) / kSkF * kSkF)) : 0;        // second v_posed buffer (pipelined blend)
   st->arena_bytes = floats * sizeof(float);
   cudaError_t e = cudaMalloc(&st->arena, st->arena_bytes);
   if (e != cudaSuccess) { free(st); return (int)e; }
@@ -753,7 +455,6 @@ extern "C" int glamr_opt_create(glamr_opt_t** out, const glamr_smpl_t* smpl, con
   st->partial = (double*)(b + o_partial);
   st->adam.beta_pow = (double*)(b + o_beta);
   st->tickets = (unsigned int*)(b + o_ticket);
-  st->kpg = (KpGrad*)(b + o_kpg);
   st->sc.heading = b + o_heading; st->sc.xy = b + o_xy; st->sc.traj_local = b + o_tl; st->sc.orient_base = b + o_ob;
   st->sc.trans_base = b + o_tb; st->sc.orient_world = b + o_ow; st->sc.trans_world = b + o_tw; st->sc.cam = b + o_cam;
   st->sc.cam_inv = b + o_caminv; st->sc.cam_d6 = b + o_camd6; st->sc.joints_world = b + o_jw; st->sc.kp_pred = b + o_kp;
@@ -762,10 +463,6 @@ extern "C" int glamr_opt_create(glamr_opt_t** out, const glamr_smpl_t* smpl, con
   st->sc.grad = nullptr;
   st->adam.m = b + o_m; st->adam.v = b + o_v;
   st->ws = smpl_carve_workspace(b + o_ws, (int)N, smpl->dev.S);
-  if (st->blend_early || st->blend_split > 0) {
-    st->ws.vpT2 = b + o_vp2;
-    st->ws.flip_src = st->adam.beta_pow + 2;
-  }
   const double one[3] = {1.0, 1.0, 0.0};
   e = cudaMemcpy(st->adam.beta_pow, one, sizeof(one), cudaMemcpyHostToDevice);
   if (e != cudaSuccess) { cudaFree(st->arena); free(st); return (int)e; }
@@ -891,19 +588,15 @@ extern "C" int glamr_opt_set_problem(glamr_opt_t* st, const glamr_problem_t* pb,
 
 extern "C" size_t glamr_opt_reduce_count(const glamr_opt_t* st) { return st ? (size_t)st->pb.n_params + GLAMR_NUM_TERMS : 0; }
 
-extern "C" int glamr_opt_launch_count(const glamr_opt_t* st, int via_iterate) {
+extern "C" int glamr_opt_launch_count(const glamr_opt_t* st) {
   if (!st) return GLAMR_EINVAL;
   const bool from_persons = st->pb.cam_mode == GLAMR_CAM_FROM_PERSONS;
   const bool has_frames = st->pb.n_end > st->pb.n_begin;
-  const int fwd = 1 + (from_persons ? 1 : 0) + (has_frames ? (st->fused ? 0 : 1) + (lbs_kernel_count(st->smpl) == 2 ? 3 : 1) : 0);     // forward [+ cam_forward] [+ pose_prep] + lbs
-  if (st->fused && !from_persons)                                        // fused tail; Adam inside it when glamr_opt_iterate runs a single-GPU loop
-    return fwd + 1 + ((via_iterate && st->peer.world <= 1) ? 0 : 1);
+  const int fwd = 1 + (from_persons ? 1 : 0) + (has_frames ? 1 + (lbs_kernel_count(st->smpl) == 2 ? 3 : 1) : 0);     // forward [+ cam_forward] [+ pose_prep + lbs]
   return fwd + 1 + (from_persons ? 2 : 0) + 1 + 1;                       // residuals [+ camera backward + scatter] + traj/cam backward + apply
 }
 
 #define GLAMR_MARK() do { if (st->timing == 2 && st->n_ev < 24) GLAMR_CUDA_TRY(cudaEventRecord(st->ev[st->n_ev++], s)); } while (0)
-
-struct FusedAdam { float* theta; double lr; float* loss_terms; int hist_stride; };
 
 // the side stream's work of an earlier evaluation whose join was left to the next call on the handle
 static int join_pending(glamr_opt_t* st, cudaStream_t s) {
@@ -916,8 +609,7 @@ static int join_pending(glamr_opt_t* st, cudaStream_t s) {
 
 // defer_join: the caller runs glamr_opt_apply on the same handle next (possibly after an exchange of reduce_buf): the pipelined blend on the
 // side stream is joined there, so that the exchange overlaps its tail instead of waiting for it
-static int backward_impl(glamr_opt_t* st, const float* theta, float* reduce_buf, void* stream, bool use_peers, const FusedAdam* adam = nullptr,
-                         bool defer_join = false) {
+static int backward_impl(glamr_opt_t* st, const float* theta, float* reduce_buf, void* stream, bool use_peers, bool defer_join = false) {
   if (!st || !theta || !reduce_buf) return GLAMR_EINVAL;
   PeerCtx pc = st->peer;
   if (!use_peers) pc.world = 0;
@@ -929,7 +621,6 @@ static int backward_impl(glamr_opt_t* st, const float* theta, float* reduce_buf,
   st->n_ev = 0;
   GLAMR_MARK();
   const glamr_problem_t& pb = st->pb;
-  const int N = pb.P * pb.T;
   OptCtx c = make_ctx(st, theta, reduce_buf);
   const bool from_persons = pb.cam_mode == GLAMR_CAM_FROM_PERSONS;
   // SMPL for the frame-persons this rank owns (global_recon_model.py:517-524); tile-major scratch (A, pf) is local to the launch
@@ -938,9 +629,6 @@ static int backward_impl(glamr_opt_t* st, const float* theta, float* reduce_buf,
   wo.jposed += (size_t)n_begin * kNJ * 3;
   wo.vcompact += (size_t)n_begin * st->smpl.S * 3;
   wo.root_raw += (size_t)n_begin * 3;
-  const int lpad = (pb.T + 31) & ~31;
-  const size_t fwd_smem = (size_t)3 * lpad * sizeof(float);
-  const bool fused_fwd = st->fused && fwd_smem <= 200 * 1024;
   const bool tc = lbs_path() >= 1 && st->smpl.tcB != nullptr;
   SmplWorkspace wo_pose = wo;
   if (tc) {
@@ -949,19 +637,6 @@ static int backward_impl(glamr_opt_t* st, const float* theta, float* reduce_buf,
       GLAMR_CUDA_TRY(cudaStreamCreateWithFlags(&st->aux, cudaStreamNonBlocking));
       GLAMR_CUDA_TRY(cudaEventCreateWithFlags(&st->ev_fork, cudaEventDisableTiming));
       GLAMR_CUDA_TRY(cudaEventCreateWithFlags(&st->ev_join, cudaEventDisableTiming));
-    }
-  }
-  {
-    static bool carve = false;
-    if (!carve && (smem_carveout_mask() & 4)) {
-      carve = true;
-      GLAMR_CUDA_TRY(cudaFuncSetAttribute(traj_cam_forward_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-      GLAMR_CUDA_TRY(cudaFuncSetAttribute(cam_forward_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-      GLAMR_CUDA_TRY(cudaFuncSetAttribute(frame_residuals_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-      GLAMR_CUDA_TRY(cudaFuncSetAttribute(camera_backward_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-      GLAMR_CUDA_TRY(cudaFuncSetAttribute(camera_scatter_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-      GLAMR_CUDA_TRY(cudaFuncSetAttribute(traj_cam_backward_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-      GLAMR_CUDA_TRY(cudaFuncSetAttribute(apply_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
     }
   }
   bool forked = false;
@@ -973,109 +648,82 @@ static int backward_impl(glamr_opt_t* st, const float* theta, float* reduce_buf,
 #endif
   const float* const pose_l = pb.smpl_pose_all + (size_t)n_begin * 69;
   const float* const beta_l = pb.smpl_beta_all + (size_t)n_begin * kNB;
-  // the blend of the NEXT evaluation (it depends on body pose / betas only): side stream, concurrent with this evaluation
-  // part 0: the whole blend; part 1: the features + the first `mt_split` frame tiles; part 2: the remaining tiles
-  const int mt_all = (n_end - n_begin + kTcM - 1) / kTcM;
-  int mt_split = -1;                            // -1: one launch sequence after the skinning; >= 0: features (+ mt_split tiles) at the top
-  if (st->blend_split > 0 && !st->timing && mt_all > 1) {
-    mt_split = (mt_all * st->blend_split + 50) / 100;
-    if (mt_split < 1) mt_split = 1;
-    if (mt_split > mt_all - 1) mt_split = mt_all - 1;
-  } else if (st->features_early && !st->timing && !st->blend_early) {
-    mt_split = 0;                               // only the (tiny) feature kernel moves to the top: the GEMM's operand is ready when the skinning ends
-  }
-  auto fork_blend = [&](int part) -> int {
-    SmplWorkspace wn = wo;
-    wn.flip_add = 1;                           // with two buffers: the one the next step's skinning will read
+  // the blend of the NEXT evaluation (it depends on body pose / betas only): side stream, concurrent with this evaluation.  With
+  // features_early its feature kernel is forked at the top and the GEMM after the skinning (which must have read v_posed first);
+  // otherwise both are forked after the skinning.
+  const int nn = n_end - n_begin;
+  const bool features_early = st->features_early && !st->timing;
+  auto fork = [&]() -> int {
     GLAMR_CUDA_TRY(cudaEventRecord(st->ev_fork, s));
     GLAMR_CUDA_TRY(cudaStreamWaitEvent(st->aux, st->ev_fork, 0));
-    if (st->timing && part != 2) GLAMR_CUDA_TRY(cudaEventRecord(st->ev_blend0, st->aux));
-    if (!(exp_skip & 1)) {
-      const int rc = launch_blend(st->smpl, n_end - n_begin, pose_l, beta_l, wn, st->aux, part == 2 ? mt_split : 0, part == 1 ? mt_split : -1, part != 2);
-      if (rc) return rc;
-    }
-    if (part != 1) {
-      if (st->timing) GLAMR_CUDA_TRY(cudaEventRecord(st->ev_blend1, st->aux));
-      GLAMR_CUDA_TRY(cudaEventRecord(st->ev_join, st->aux));
-      forked = true;
-    }
     return GLAMR_OK;
   };
-  if (tc && n_end > n_begin) {
-    if (!st->vpt_ready) {                 // first evaluation after create / a new sequence: the current buffer is filled in order
-      const int rc = launch_blend(st->smpl, n_end - n_begin, pose_l, beta_l, wo, s);
-      if (rc) return rc;
+  if (tc && nn > 0) {
+    int rc;
+    if (!st->vpt_ready) {                 // first evaluation after create / a new sequence: v_posed is filled in order
+      if ((rc = launch_blend(st->smpl, nn, pose_l, beta_l, wo, s))) return rc;
       st->vpt_ready = 1;
     }
-    if (st->blend_early || mt_split >= 0) {
-      const int rc = fork_blend(st->blend_early ? 0 : 1);
-      if (rc) return rc;
+    if (features_early) {
+      if ((rc = fork())) return rc;
+      if (!(exp_skip & 1))
+        if ((rc = launch_blend_features(nn, pose_l, beta_l, wo, st->aux))) return rc;
     }
   }
-  if (fused_fwd) {
-    if (fwd_smem > 48 * 1024 && st->fwd_smem_set < fwd_smem) {
-      GLAMR_CUDA_TRY(cudaFuncSetAttribute(forward_pose_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)fwd_smem));
-      st->fwd_smem_set = fwd_smem;
-    }
-    const int chunks = (pb.T + kFwdFrames - 1) / kFwdFrames;
-    GLAMR_CUDA_TRY(launch_pdl(1, forward_pose_kernel, dim3(pb.P * chunks), dim3(kScanThreads), fwd_smem, s, c, st->smpl, wo_pose, n_begin,
-                              from_persons ? 0 : 1, chunks, lpad));      // also zeroes reduce_buf
-  } else {
-    GLAMR_CUDA_TRY(launch_pdl(1, traj_cam_forward_kernel, dim3(pb.P + st->cam_blocks), dim3(kScanThreads), 0, s, c, from_persons ? 0 : 1));   // also zeroes reduce_buf
-  }
+  traj_cam_forward_kernel<<<pb.P + st->cam_blocks, kScanThreads, 0, s>>>(c, from_persons ? 0 : 1);   // also zeroes reduce_buf
+  GLAMR_LAUNCH_CHECK();
   GLAMR_MARK();
   if (from_persons) {          // the camera is the mean of the persons' world transforms: needs traj_forward of all persons
-    GLAMR_CUDA_TRY(launch_pdl(1, cam_forward_kernel, dim3(st->slots_cam), dim3(kFrameThreads), 0, s, c));
+    cam_forward_kernel<<<st->slots_cam, kFrameThreads, 0, s>>>(c);
+    GLAMR_LAUNCH_CHECK();
   }
   GLAMR_MARK();
-  if (n_end > n_begin) {
-    const int nn = n_end - n_begin;
+  if (nn > 0) {
     int rc;
-    if (!fused_fwd)
-      if ((rc = launch_pose_prep(st->smpl, nn, st->sc.orient_world + (size_t)n_begin * 3, pose_l, beta_l, 1, wo_pose, s, true))) return rc;
+    if ((rc = launch_pose_prep(st->smpl, nn, st->sc.orient_world + (size_t)n_begin * 3, pose_l, beta_l, 1, wo_pose, s))) return rc;
     GLAMR_MARK();
+    if (st->timing) GLAMR_CUDA_TRY(cudaEventRecord(st->ev_lbs0, s));
     if (tc) {
-      if (st->timing) GLAMR_CUDA_TRY(cudaEventRecord(st->ev_lbs0, s));
       if (!(exp_skip & 2))
         if ((rc = launch_skin(st->smpl, nn, wo, nullptr, s))) return rc;
       if (st->timing) GLAMR_CUDA_TRY(cudaEventRecord(st->ev_lbs1, s));
-      if (!st->blend_early)                 // the (rest of the) next blend: with a single buffer it may only start once this skinning has read v_posed
-        if ((rc = fork_blend(mt_split >= 0 ? 2 : 0))) return rc;
+      if ((rc = fork())) return rc;
+      if (st->timing) GLAMR_CUDA_TRY(cudaEventRecord(st->ev_blend0, st->aux));
+      if (!(exp_skip & 1)) {
+        if (!features_early)
+          if ((rc = launch_blend_features(nn, pose_l, beta_l, wo, st->aux))) return rc;
+        if ((rc = launch_blend_gemm(st->smpl, nn, wo, st->aux))) return rc;
+      }
+      if (st->timing) GLAMR_CUDA_TRY(cudaEventRecord(st->ev_blend1, st->aux));
+      GLAMR_CUDA_TRY(cudaEventRecord(st->ev_join, st->aux));
+      forked = true;
     } else {
-      if (st->timing) GLAMR_CUDA_TRY(cudaEventRecord(st->ev_lbs0, s));
-      if ((rc = launch_lbs(st->smpl, 0, nn, beta_l, wo, nullptr, s, true))) return rc;
+      if ((rc = launch_lbs(st->smpl, 0, nn, beta_l, wo, nullptr, s))) return rc;
       if (st->timing) GLAMR_CUDA_TRY(cudaEventRecord(st->ev_lbs1, s));
     }
     GLAMR_MARK();
   }
-  if (st->fused && !from_persons) {
-    FusedArgs a;
-    a.kpg = st->kpg; a.partial = st->partial; a.person_ticket = st->tickets + 4; a.global_ticket = st->tickets + 2;
-    a.reduce_buf = reduce_buf; a.ad = st->adam;
-    a.theta = adam ? adam->theta : nullptr; a.lr = adam ? adam->lr : 0.0; a.loss_terms = adam ? adam->loss_terms : nullptr;
-    a.hist_stride = adam ? adam->hist_stride : 0; a.do_adam = adam ? 1 : 0;
-    GLAMR_CUDA_TRY(launch_pdl(8, residuals_backward_kernel, dim3((N + kFusedFramesPerCta - 1) / kFusedFramesPerCta), dim3(kScanThreads), 0, s, c, st->smpl, wo,
-                              n_begin, a));
-    GLAMR_MARK();
-    if (forked) GLAMR_CUDA_TRY(cudaStreamWaitEvent(s, st->ev_join, 0));
-    return GLAMR_OK;
-  }
-  if (adam) return GLAMR_EINVAL;               // Adam inside the backward pass exists only in the fused kernel
   double* part_res = st->partial;
   double* part_traj = st->partial + (size_t)st->slots_res * GLAMR_NUM_TERMS;
   double* part_cam3 = part_traj + (size_t)(pb.P + st->cam_blocks) * GLAMR_NUM_TERMS;
-  if (!(exp_skip & 4))
-    GLAMR_CUDA_TRY(launch_pdl(8, frame_residuals_kernel, dim3(st->slots_res), dim3(kFrameThreads), 0, s, c, st->smpl, wo, n_begin, part_res));
+  if (!(exp_skip & 4)) {
+    frame_residuals_kernel<<<st->slots_res, kFrameThreads, 0, s>>>(c, st->smpl, wo, n_begin, part_res);
+    GLAMR_LAUNCH_CHECK();
+  }
   GLAMR_MARK();
   if (from_persons) {
-    GLAMR_CUDA_TRY(launch_pdl(16, camera_backward_kernel, dim3(st->slots_cam), dim3(kFrameThreads), 0, s, c, part_cam3));
-    GLAMR_CUDA_TRY(launch_pdl(16, camera_scatter_kernel, dim3(st->slots_cam), dim3(kFrameThreads), 0, s, c));
+    camera_backward_kernel<<<st->slots_cam, kFrameThreads, 0, s>>>(c, part_cam3);
+    GLAMR_LAUNCH_CHECK();
+    camera_scatter_kernel<<<st->slots_cam, kFrameThreads, 0, s>>>(c);
+    GLAMR_LAUNCH_CHECK();
     GLAMR_MARK();
   }
   const int n_slots = st->slots_res + pb.P + st->cam_blocks + (from_persons ? st->slots_cam : 0);
-  if (!(exp_skip & 8))
-    GLAMR_CUDA_TRY(launch_pdl(16, traj_cam_backward_kernel, dim3(pb.P + st->cam_blocks), dim3(kScanThreads), 0, s, c, from_persons ? 0 : 1, part_traj,
-                              (const double*)st->partial, n_slots, reduce_buf, st->tickets, pc));
+  if (!(exp_skip & 8)) {
+    traj_cam_backward_kernel<<<pb.P + st->cam_blocks, kScanThreads, 0, s>>>(c, from_persons ? 0 : 1, part_traj, (const double*)st->partial, n_slots,
+                                                                            reduce_buf, st->tickets, pc);
+    GLAMR_LAUNCH_CHECK();
+  }
   GLAMR_MARK();
   if (forked) {
     if (defer_join) st->join_pending = 1;
@@ -1090,7 +738,7 @@ extern "C" int glamr_opt_backward(glamr_opt_t* st, const float* theta, float* re
 // between): same work as glamr_opt_backward, but the side-stream blend of the next evaluation is joined by that apply call (or by the next
 // call on the handle), so the exchange runs next to its tail.
 extern "C" int glamr_opt_backward_for_apply(glamr_opt_t* st, const float* theta, float* reduce_buf, void* stream) {
-  return backward_impl(st, theta, reduce_buf, stream, false, nullptr, true);
+  return backward_impl(st, theta, reduce_buf, stream, false, true);
 }
 
 extern "C" int glamr_opt_losses(glamr_opt_t* st, const float* reduce_buf, float* loss_terms, void* stream) {
@@ -1113,8 +761,8 @@ static int apply_impl(glamr_opt_t* st, float* theta, const float* reduce_buf, do
   }
   OptCtx c = make_ctx(st, theta, nullptr);
   const int blocks = (st->pb.n_params + 255) / 256;
-  GLAMR_CUDA_TRY(launch_pdl(32, apply_kernel, dim3(blocks < 296 ? blocks : 296), dim3(256), 0, s, c, theta, reduce_buf, lr, st->adam, loss_terms,
-                            loss_hist_stride, st->tickets + 1, pc));
+  apply_kernel<<<blocks < 296 ? blocks : 296, 256, 0, s>>>(c, theta, reduce_buf, lr, st->adam, loss_terms, loss_hist_stride, st->tickets + 1, pc);
+  GLAMR_LAUNCH_CHECK();
   GLAMR_MARK();
   return GLAMR_OK;
 }
@@ -1191,12 +839,7 @@ extern "C" int glamr_opt_iterate(glamr_opt_t* st, float* theta, float* reduce_bu
   cudaStream_t s = (cudaStream_t)stream;
   int rc, done = 0;
   const bool peers = st->peer.world > 1;      // W > 1: backward publishes, apply sums the peers' slots (no call in between)
-  const bool fused_adam = st->fused && !peers && st->pb.cam_mode != GLAMR_CAM_FROM_PERSONS;
   auto eager = [&](cudaStream_t q) -> int {
-    if (fused_adam) {
-      const FusedAdam fa = {theta, lr, loss_terms, loss_hist_stride};
-      return backward_impl(st, theta, reduce_buf, q, false, &fa);
-    }
     if ((rc = backward_impl(st, theta, reduce_buf, q, peers))) return rc;
     return apply_impl(st, theta, reduce_buf, lr, loss_terms, loss_hist_stride, q, peers);
   };

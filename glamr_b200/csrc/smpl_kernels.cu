@@ -21,8 +21,6 @@ namespace glamr {
 __global__ void __launch_bounds__(128) pose_prep_kernel(SmplDev m, int n, const float* __restrict__ orient,
                                                         const float* __restrict__ body_pose,
                                                         const float* __restrict__ betas, int use_betas, SmplWorkspace w) {
-  pdl_launch_dependents();
-  pdl_wait();
   const int f = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   if (f >= n) return;
   pose_prep_frame(m, f, orient ? orient + (size_t)f * 3 : nullptr, body_pose + (size_t)f * 69, use_betas ? betas + (size_t)f * kNB : nullptr, w,
@@ -77,7 +75,6 @@ lbs_kernel(SmplDev m, int n_begin, int n_end, const float* __restrict__ betas, S
   const float* pd_slab = m.pd_tiles + (size_t)vtile * kPF * kTileCols;
   const float* pf_slab = w.pf + (size_t)(f0 >> 5) * kNChunks * kPfChunkFloats;
 
-  pdl_launch_dependents();
   // issue the per-vertex constant loads first: their latency overlaps the barrier set-up and the first TMA round trip
   float sdv[kVertsPerThread][30], vt[kVertsPerThread][3];
   {
@@ -118,8 +115,7 @@ lbs_kernel(SmplDev m, int n_begin, int n_end, const float* __restrict__ betas, S
     tma_bulk_g2s(PDs + s * kChunkFloats, pd_slab + (size_t)c * kChunkFloats, kChunkBytes, &full[s]);
     tma_bulk_g2s(pfs + s * kPfChunkFloats, pf_slab + (size_t)c * kPfChunkFloats, kPfChunkBytes, &full[s]);
   };
-  // posedirs is a model constant: the first stages' slabs are fetched before this grid waits for its producer
-  // (pose_prep_kernel, PDL); their pose-feature halves and the A tile follow after pdl_wait().
+  // the first stages' posedirs slabs are requested here; their pose-feature halves and the A tile follow the shape blend below
   if (tid == 0) {
 #pragma unroll
     for (int c = 0; c < kStages - 1; ++c) {
@@ -154,7 +150,6 @@ lbs_kernel(SmplDev m, int n_begin, int n_end, const float* __restrict__ betas, S
     }
   }
 
-  pdl_wait();                          // A and pf below are written by pose_prep_kernel
   if (tid == 0) {
     mbar_expect_tx(abar, (uint32_t)kATileFloats * sizeof(float));
     tma_bulk_g2s(As, w.A + (size_t)(f0 >> 5) * kATileFloats, (uint32_t)kATileFloats * sizeof(float), abar);
@@ -347,7 +342,7 @@ constexpr uint32_t kTcABytes = kTcAStageFloats * sizeof(float);      // 8,192
 constexpr uint32_t kTcBBytes = kTcBStageFloats * sizeof(float);      // 16,384
 constexpr size_t kTcSmemBytes = (size_t)kTcStages * (kTcABytes + kTcBBytes) + 128;
 
-__global__ void __launch_bounds__(kTcThreads) lbs_blend_tc_kernel(SmplDev m, SmplWorkspace w, int mtile0) {
+__global__ void __launch_bounds__(kTcThreads) lbs_blend_tc_kernel(SmplDev m, SmplWorkspace w) {
   extern __shared__ __align__(128) unsigned char tc_raw[];
   float* As = reinterpret_cast<float*>(tc_raw);                                   // [stages][hi | lo][2][128][4]
   float* Bs = As + kTcStages * kTcAStageFloats;                                   // [stages][hi | lo][2][256][4]
@@ -356,8 +351,7 @@ __global__ void __launch_bounds__(kTcThreads) lbs_blend_tc_kernel(SmplDev m, Smp
   uint64_t* acc_full = empty + kTcStages;
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(acc_full + 1);
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  const int ntile = blockIdx.x, mtile = blockIdx.y + mtile0;     // mtile0: first 128-frame tile of this launch (the optimiser splits the blend in two launches)
-  pdl_launch_dependents();
+  const int ntile = blockIdx.x, mtile = blockIdx.y;
   if (warp == 1) {
     asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "r"(kTcN));
     asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::);
@@ -377,12 +371,10 @@ __global__ void __launch_bounds__(kTcThreads) lbs_blend_tc_kernel(SmplDev m, Smp
     if (lane == 0) {
       const float* gA = w.tcA + (size_t)mtile * kTcChunks * kTcAStageFloats;
       const float* gB = m.tcB + (size_t)ntile * kTcChunks * kTcBStageFloats;
-      // the basis is a model constant: its first stages are requested before this grid waits for the kernel that writes the features
       for (int c = 0; c < kTcStages; ++c) {
         mbar_expect_tx_only(&full[c], kTcBBytes);
         tma_bulk_g2s(Bs + c * kTcBStageFloats, gB + (size_t)c * kTcBStageFloats, kTcBBytes, &full[c]);
       }
-      pdl_wait();
       for (int c = 0; c < kTcChunks; ++c) {
         const int s = c % kTcStages;
         if (c >= kTcStages) {
@@ -422,9 +414,8 @@ __global__ void __launch_bounds__(kTcThreads) lbs_blend_tc_kernel(SmplDev m, Smp
     const int q = warp & 3;
     const int frame = mtile * kTcM + q * 32 + lane;                              // < w.mpad by construction
     // v_posed^T [column][frame], or frame-tiled [frame / 20][column][frame % 20] for the tensor-core skinning
-    float* const vpb = vp_buffer(w);
-    float* out = w.vp_tiled ? vpb + ((size_t)(frame / kSkF) * kTcCols + (size_t)ntile * kTcN) * kSkF + frame % kSkF
-                            : vpb + (size_t)ntile * kTcN * w.mpad + frame;
+    float* out = w.vp_tiled ? w.vpT + ((size_t)(frame / kSkF) * kTcCols + (size_t)ntile * kTcN) * kSkF + frame % kSkF
+                            : w.vpT + (size_t)ntile * kTcN * w.mpad + frame;
     const size_t cstride = w.vp_tiled ? (size_t)kSkF : (size_t)w.mpad;
 #pragma unroll 1
     for (int cc = 0; cc < kTcN / 32; ++cc) {
@@ -462,7 +453,6 @@ __global__ void __launch_bounds__(kLbsThreads) lbs_skin_kernel(SmplDev m, int n_
   const int tid = threadIdx.x, lane = tid & 31;
   const int vtile = blockIdx.x;
   const int f0 = n_begin + blockIdx.y * kFramesPerCta;
-  pdl_launch_dependents();
   if (tid == 0) {
     mbar_init(abar, 1);
     mbar_fence_init();
@@ -477,7 +467,6 @@ __global__ void __launch_bounds__(kLbsThreads) lbs_skin_kernel(SmplDev m, int n_
     my_j = *reinterpret_cast<const unsigned int*>(m.skin_j + (size_t)gvl * 4);
   }
   const int my_ci = m.compact_of_vertex[gvl];
-  pdl_wait();                                   // A (pose_prep) and vpT (blend GEMM) are written by preceding kernels
   if (tid == 0) {
     mbar_expect_tx(abar, (uint32_t)kATileFloats * sizeof(float));
     tma_bulk_g2s(As, w.A + (size_t)(f0 >> 5) * kATileFloats, (uint32_t)kATileFloats * sizeof(float), abar);
@@ -485,8 +474,8 @@ __global__ void __launch_bounds__(kLbsThreads) lbs_skin_kernel(SmplDev m, int n_
   const int fr = lane;
   const int n = f0 + fr;
   const bool n_ok = n < n_end;
-  const float* vp = vp_buffer(w) + (size_t)(vtile * kVTile + vbase) * 3 * w.mpad + n;      // n < mpad (frames padded to 128)
   mbar_wait(abar, 0);
+  const float* vp = w.vpT + (size_t)(vtile * kVTile + vbase) * 3 * w.mpad + n;      // n < mpad (frames padded to 128)
   constexpr int U = 4;
 #pragma unroll 1
   for (int i0 = 0; i0 < 32; i0 += U) {
@@ -598,7 +587,6 @@ __global__ void __launch_bounds__(kSkinTcThreads) lbs_skin_tc_kernel(SmplDev m, 
   const int vtile = blockIdx.x;
   const int ftile0 = blockIdx.y * kSkTilesPerCta;
   const int ntiles = min(kSkTilesPerCta, (n + kSkF - 1) / kSkF - ftile0);
-  pdl_launch_dependents();
   if (warp == 1) {
     asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "r"(256));
     asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::);
@@ -621,9 +609,7 @@ __global__ void __launch_bounds__(kSkinTcThreads) lbs_skin_tc_kernel(SmplDev m, 
   if (warp == 0) {
     if (lane == 0) {
       mbar_expect_tx(full_w, kSkWBytes);
-      tma_bulk_g2s(Ws, m.skW + (size_t)vtile * kSkWImageFloats, kSkWBytes, full_w);          // model constant: before the dependency wait
-      pdl_wait();                                                                           // skB (pose prep) and v_posed (blend) below
-      const float* const vpb = vp_buffer(w);
+      tma_bulk_g2s(Ws, m.skW + (size_t)vtile * kSkWImageFloats, kSkWBytes, full_w);
       for (int it = 0; it < ntiles; ++it) {
         const int ftile = ftile0 + it;
         if (it > 0) mbar_wait(b_empty, (it - 1) & 1);
@@ -631,7 +617,7 @@ __global__ void __launch_bounds__(kSkinTcThreads) lbs_skin_tc_kernel(SmplDev m, 
         tma_bulk_g2s(Bs, w.skB + (size_t)ftile * kSkBImageFloats, kSkBBytes, full_b);
         if (it > 0) mbar_wait(v_empty, (it - 1) & 1);
         mbar_expect_tx(full_v, kSkVBytes);
-        tma_bulk_g2s(Vs, vpb + ((size_t)ftile * kTcCols + (size_t)vtile * kTileCols) * kSkF, kSkVBytes, full_v);
+        tma_bulk_g2s(Vs, w.vpT + ((size_t)ftile * kTcCols + (size_t)vtile * kTileCols) * kSkF, kSkVBytes, full_v);
       }
     }
   } else if (warp == 1) {
@@ -773,47 +759,27 @@ __global__ void fk24_finalize_kernel(int n, const float* __restrict__ jposed, co
 
 // ------------------------------------------------------------------------------------------------ launches
 int launch_pose_prep(const SmplDev& m, int n, const float* orient, const float* body_pose, const float* betas, int use_betas,
-                     const SmplWorkspace& w, cudaStream_t s, bool pdl) {
+                     const SmplWorkspace& w, cudaStream_t s) {
   if (n <= 0) return GLAMR_OK;
-  const int blocks = (n + 3) / 4;
-  if (pdl) {
-    GLAMR_CUDA_TRY(launch_pdl(2, pose_prep_kernel, dim3(blocks), dim3(128), 0, s, m, n, orient, body_pose, betas, use_betas, w));
-    return GLAMR_OK;
-  }
-  pose_prep_kernel<<<blocks, 128, 0, s>>>(m, n, orient, body_pose, betas, use_betas, w);
+  pose_prep_kernel<<<(n + 3) / 4, 128, 0, s>>>(m, n, orient, body_pose, betas, use_betas, w);
   GLAMR_LAUNCH_CHECK();
   return GLAMR_OK;
 }
 
-// pdl: launch with the programmatic-serialization attribute.  Only for callers whose betas are long-lived constants
-// (the optimiser): the kernel reads betas / shapedirs / posedirs BEFORE it waits for the preceding grid.
 // An SM runs with ONE L1 / shared-memory split at a time.  blend_features_kernel / pose_prep_kernel have no dynamic shared memory, so by
 // default they run with a small shared-memory split, and the GEMM kernel that follows each of them in its stream (2 x 96-101 KB per SM)
 // can only be placed on an SM after the small kernel's CTAs have drained and the SM has been re-configured.  Asking for the maximal
 // shared-memory split on the small SMPL kernels too removes that hand-over: 193.0 -> 157.4 us per iteration at 4 x 300 frame-persons
-// (no change at 1 x 300).  The optimiser's own small kernels lose more from the smaller L1 than they gain (bit 4: +6 us at 1 x 300).
-// GLAMR_SMEM_CARVEOUT bit mask: which kernels ask for the maximal shared-memory split (cudaFuncAttributePreferredSharedMemoryCarveout):
-// 1 = the two LBS GEMM kernels, 2 = the small SMPL kernels next to them, 4 = the optimiser's small kernels (globalopt_kernels.cu)
-int smem_carveout_mask() {
-  static int v = -1;
-  if (v < 0) {
-    const char* e = getenv("GLAMR_SMEM_CARVEOUT");
-    v = e ? atoi(e) : GLAMR_DEFAULT_SMEM_CARVEOUT;
-  }
-  return v;
-}
+// (no change at 1 x 300).  The optimiser's own small kernels lose more from the smaller L1 than they gain (+6 us at 1 x 300), so they
+// keep the default split.
 static int lbs_set_attrs() {
   static bool attrs = false;
   if (!attrs) {
     attrs = true;
-    if (smem_carveout_mask() & 1) {
-      GLAMR_CUDA_TRY(cudaFuncSetAttribute(lbs_blend_tc_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-      GLAMR_CUDA_TRY(cudaFuncSetAttribute(lbs_skin_tc_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-    }
-    if (smem_carveout_mask() & 2) {
-      GLAMR_CUDA_TRY(cudaFuncSetAttribute(blend_features_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-      GLAMR_CUDA_TRY(cudaFuncSetAttribute(pose_prep_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-    }
+    GLAMR_CUDA_TRY(cudaFuncSetAttribute(lbs_blend_tc_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+    GLAMR_CUDA_TRY(cudaFuncSetAttribute(lbs_skin_tc_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+    GLAMR_CUDA_TRY(cudaFuncSetAttribute(blend_features_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+    GLAMR_CUDA_TRY(cudaFuncSetAttribute(pose_prep_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
     GLAMR_CUDA_TRY(cudaFuncSetAttribute(lbs_blend_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kTcSmemBytes));
     GLAMR_CUDA_TRY(cudaFuncSetAttribute(lbs_skin_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSkinSmemBytes));
     GLAMR_CUDA_TRY(cudaFuncSetAttribute(lbs_skin_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSkinSmemBytes));
@@ -821,24 +787,28 @@ static int lbs_set_attrs() {
   }
   return GLAMR_OK;
 }
-// blend features + blend GEMM for local frame-persons [0, n): v_posed (transposed) of the workspace
-// mt_begin / mt_end: the range of 128-frame tiles of the GEMM this call launches (mt_end < 0: all); features: also (re)build the A operand
-int launch_blend(const SmplDev& m, int n, const float* body_pose, const float* betas, const SmplWorkspace& w, cudaStream_t s, int mt_begin,
-                 int mt_end, bool features) {
+// the A operand of the blend GEMM for local frame-persons [0, n)
+int launch_blend_features(int n, const float* body_pose, const float* betas, const SmplWorkspace& w, cudaStream_t s) {
   if (n <= 0) return GLAMR_OK;
   int rc;
   if ((rc = lbs_set_attrs())) return rc;
-  const int mtiles = (n + kTcM - 1) / kTcM;
-  if (mt_end < 0 || mt_end > mtiles) mt_end = mtiles;
-  if (features) {
-    blend_features_kernel<<<(n + 3) / 4, 128, 0, s>>>(n, body_pose, betas, w);
-    GLAMR_LAUNCH_CHECK();
-  }
-  if (mt_end > mt_begin) {
-    lbs_blend_tc_kernel<<<dim3(kTcNTiles, mt_end - mt_begin), kTcThreads, kTcSmemBytes, s>>>(m, w, mt_begin);
-    GLAMR_LAUNCH_CHECK();
-  }
+  blend_features_kernel<<<(n + 3) / 4, 128, 0, s>>>(n, body_pose, betas, w);
+  GLAMR_LAUNCH_CHECK();
   return GLAMR_OK;
+}
+// blend GEMM for local frame-persons [0, n) from the workspace's features: v_posed (transposed) of the workspace
+int launch_blend_gemm(const SmplDev& m, int n, const SmplWorkspace& w, cudaStream_t s) {
+  if (n <= 0) return GLAMR_OK;
+  int rc;
+  if ((rc = lbs_set_attrs())) return rc;
+  lbs_blend_tc_kernel<<<dim3(kTcNTiles, (n + kTcM - 1) / kTcM), kTcThreads, kTcSmemBytes, s>>>(m, w);
+  GLAMR_LAUNCH_CHECK();
+  return GLAMR_OK;
+}
+int launch_blend(const SmplDev& m, int n, const float* body_pose, const float* betas, const SmplWorkspace& w, cudaStream_t s) {
+  int rc;
+  if ((rc = launch_blend_features(n, body_pose, betas, w, s))) return rc;
+  return launch_blend_gemm(m, n, w, s);
 }
 // skinning of local frame-persons [0, n) from the workspace's v_posed and A
 int launch_skin(const SmplDev& m, int n, const SmplWorkspace& w, float* vertices, cudaStream_t s) {
@@ -867,8 +837,7 @@ int lbs_path() {
 }
 int lbs_kernel_count(const SmplDev& m) { return (lbs_path() >= 1 && m.tcB) ? 2 : 1; }
 
-int launch_lbs(const SmplDev& m, int n_begin, int n_end, const float* betas, const SmplWorkspace& w, float* vertices, cudaStream_t s,
-               bool pdl) {
+int launch_lbs(const SmplDev& m, int n_begin, int n_end, const float* betas, const SmplWorkspace& w, float* vertices, cudaStream_t s) {
   if (n_end <= n_begin) return GLAMR_OK;
   if (n_begin % kFramesPerCta != 0) return GLAMR_EINVAL;   // the tile-major scratch is indexed by whole frame tiles
   dim3 grid(kNVTiles, (n_end - n_begin + kFramesPerCta - 1) / kFramesPerCta);
@@ -879,56 +848,34 @@ int launch_lbs(const SmplDev& m, int n_begin, int n_end, const float* betas, con
   }
   if (path >= 1 && m.tcB && w.tcA && n_begin == 0) {
     const int mtiles = (n_end + kTcM - 1) / kTcM;
+    lbs_blend_tc_kernel<<<dim3(kTcNTiles, mtiles), kTcThreads, kTcSmemBytes, s>>>(m, w);
+    GLAMR_LAUNCH_CHECK();
     if (w.vp_tiled) {
       const dim3 sgrid(kNVTiles, ((n_end + kSkF - 1) / kSkF + kSkTilesPerCta - 1) / kSkTilesPerCta);
-      if (pdl) {
-        GLAMR_CUDA_TRY(launch_pdl(4, lbs_blend_tc_kernel, dim3(kTcNTiles, mtiles), dim3(kTcThreads), kTcSmemBytes, s, m, w, 0));
-        GLAMR_CUDA_TRY(launch_pdl(4, lbs_skin_tc_kernel, sgrid, dim3(kSkinTcThreads), kSkinTcSmemBytes, s, m, n_end, w, vertices));
-      } else {
-        lbs_blend_tc_kernel<<<dim3(kTcNTiles, mtiles), kTcThreads, kTcSmemBytes, s>>>(m, w, 0);
-        GLAMR_LAUNCH_CHECK();
-        lbs_skin_tc_kernel<<<sgrid, kSkinTcThreads, kSkinTcSmemBytes, s>>>(m, n_end, w, vertices);
-        GLAMR_LAUNCH_CHECK();
-      }
-      return GLAMR_OK;
-    }
-    if (pdl) {
-      GLAMR_CUDA_TRY(launch_pdl(4, lbs_blend_tc_kernel, dim3(kTcNTiles, mtiles), dim3(kTcThreads), kTcSmemBytes, s, m, w, 0));
-      if (m.K == 4) GLAMR_CUDA_TRY(launch_pdl(4, lbs_skin_kernel<4>, grid, dim3(kLbsThreads), kSkinSmemBytes, s, m, n_begin, n_end, w, vertices));
-      else GLAMR_CUDA_TRY(launch_pdl(4, lbs_skin_kernel<0>, grid, dim3(kLbsThreads), kSkinSmemBytes, s, m, n_begin, n_end, w, vertices));
+      lbs_skin_tc_kernel<<<sgrid, kSkinTcThreads, kSkinTcSmemBytes, s>>>(m, n_end, w, vertices);
+    } else if (m.K == 4) {
+      lbs_skin_kernel<4><<<grid, kLbsThreads, kSkinSmemBytes, s>>>(m, n_begin, n_end, w, vertices);
     } else {
-      lbs_blend_tc_kernel<<<dim3(kTcNTiles, mtiles), kTcThreads, kTcSmemBytes, s>>>(m, w, 0);
-      GLAMR_LAUNCH_CHECK();
-      if (m.K == 4) lbs_skin_kernel<4><<<grid, kLbsThreads, kSkinSmemBytes, s>>>(m, n_begin, n_end, w, vertices);
-      else lbs_skin_kernel<0><<<grid, kLbsThreads, kSkinSmemBytes, s>>>(m, n_begin, n_end, w, vertices);
-      GLAMR_LAUNCH_CHECK();
+      lbs_skin_kernel<0><<<grid, kLbsThreads, kSkinSmemBytes, s>>>(m, n_begin, n_end, w, vertices);
     }
+    GLAMR_LAUNCH_CHECK();
     return GLAMR_OK;
   }
-  static int stages = 0, dbg = 0;
-  if (!stages) {
-    const char* e = getenv("GLAMR_LBS_STAGES");
-    stages = (e && atoi(e) == 4) ? 4 : 3;
+  static bool attrs = false;
+  static int dbg = 0;
+  if (!attrs) {
+    attrs = true;
 #ifdef GLAMR_EXPERIMENT
     const char* d = getenv("GLAMR_LBS_DEBUG");      // experiment build only: bit0 skips the FMA loop, bit1 the skinning phase
     dbg = d ? atoi(d) : 0;
 #endif
     GLAMR_CUDA_TRY(cudaFuncSetAttribute(lbs_kernel<4, 3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)lbs_smem_bytes(3)));
     GLAMR_CUDA_TRY(cudaFuncSetAttribute(lbs_kernel<0, 3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)lbs_smem_bytes(3)));
-    GLAMR_CUDA_TRY(cudaFuncSetAttribute(lbs_kernel<4, 4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)lbs_smem_bytes(4)));
   }
-  auto go = [&](auto kernel, size_t smem) -> int {
-    if (pdl) {
-      GLAMR_CUDA_TRY(launch_pdl(4, kernel, grid, dim3(kLbsThreads), smem, s, m, n_begin, n_end, betas, w, vertices, dbg));
-    } else {
-      kernel<<<grid, kLbsThreads, smem, s>>>(m, n_begin, n_end, betas, w, vertices, dbg);
-      GLAMR_LAUNCH_CHECK();
-    }
-    return GLAMR_OK;
-  };
-  if (m.K == 4 && stages == 4) return go(lbs_kernel<4, 4>, lbs_smem_bytes(4));
-  if (m.K == 4) return go(lbs_kernel<4, 3>, lbs_smem_bytes(3));
-  return go(lbs_kernel<0, 3>, lbs_smem_bytes(3));
+  if (m.K == 4) lbs_kernel<4, 3><<<grid, kLbsThreads, lbs_smem_bytes(3), s>>>(m, n_begin, n_end, betas, w, vertices, dbg);
+  else lbs_kernel<0, 3><<<grid, kLbsThreads, lbs_smem_bytes(3), s>>>(m, n_begin, n_end, betas, w, vertices, dbg);
+  GLAMR_LAUNCH_CHECK();
+  return GLAMR_OK;
 }
 
 int launch_joints_finalize(const SmplDev& m, int n, int orig_joints, const float* root_trans, const float* root_scale,

@@ -49,11 +49,6 @@ struct SmplWorkspace {
   int mpad;         // frames padded to a multiple of 128
   float* skB;       // [ceil(mpad/20)][hi | lo][6 joint groups][20 frames x 12][4]  the relative joint transforms as the B operand of the
                     //              tensor-core skinning (row = frame-in-tile * 12 + element of the 3x4, K = joint), tf32 hi / lo
-  float* vpT2;      // optimiser only: second v_posed buffer (same layout as vpT) or NULL.  The blend of evaluation i + 1 is launched while
-                    //              evaluation i still reads v_posed, so the two alternate: buffer = (step + flip_add) & 1 with the Adam step
-                    //              count read from device memory (*flip_src), which keeps one captured graph valid for every iteration
-  const double* flip_src;
-  int flip_add;     // 0: the buffer of the current step (skinning, in-order blend), 1: the buffer of the next step (pipelined blend)
   int vp_tiled;     // 1: v_posed is stored frame-tiled for lbs_skin_tc_kernel: [ceil(mpad/20)][20736 cols][20 frames] (the 128 vertices x
                     //    20 frames of a skinning tile are one contiguous 30,720 B block = one bulk copy); 0: vpT as described above
 };
@@ -85,16 +80,10 @@ inline SmplWorkspace smpl_carve_workspace(void* base, int n, int S) {
   w.skB = p; p += (size_t)((w.mpad + kSkF - 1) / kSkF) * kSkBImageFloats;
   w.vpT = p;                                   // [20736][mpad] or, frame-tiled, [ceil(mpad/20)][20736][20]
   w.vp_tiled = lbs_path() == 2 ? 1 : 0;
-  w.vpT2 = nullptr; w.flip_src = nullptr; w.flip_add = 0;
   return w;
 }
 
 #if defined(__CUDACC__)
-// the v_posed buffer this launch works on (see SmplWorkspace::vpT2)
-__device__ __forceinline__ float* vp_buffer(const SmplWorkspace& w) {
-  if (!w.vpT2) return w.vpT;
-  return ((((int)*w.flip_src) + w.flip_add) & 1) ? w.vpT2 : w.vpT;
-}
 // un-rooted joint `idx` of [24 LBS | picks | extra regressed] for local frame-person f  (lib/models/smpl.py:299-301)
 __device__ __forceinline__ void raw_joint(const SmplDev& m, const SmplWorkspace& w, int f, int idx, float* o) {
   if (idx < kNJ) {
@@ -232,15 +221,16 @@ __device__ __forceinline__ void pose_prep_frame(const SmplDev& m, int f, const f
 // launches (smpl_kernels.cu); all asynchronous on `s`
 // orient may be NULL (zeros).  use_betas == 0 -> rest joints from the template only (SMPL.get_joints).
 int launch_pose_prep(const SmplDev& m, int n, const float* orient, const float* body_pose, const float* betas,
-                     int use_betas, const SmplWorkspace& w, cudaStream_t s, bool pdl = false);
+                     int use_betas, const SmplWorkspace& w, cudaStream_t s);
 // n_begin..n_end: frame-person range to skin.  vertices may be NULL.
 int launch_lbs(const SmplDev& m, int n_begin, int n_end, const float* betas, const SmplWorkspace& w, float* vertices,
-               cudaStream_t s, bool pdl = false);
-// tensor-core path in two halves (the optimiser pipelines them: the blend depends on body pose / betas only)
-int launch_blend(const SmplDev& m, int n, const float* body_pose, const float* betas, const SmplWorkspace& w, cudaStream_t s, int mt_begin = 0,
-                 int mt_end = -1, bool features = true);
+               cudaStream_t s);
+// tensor-core path in parts (the optimiser pipelines them: the blend depends on body pose / betas only):
+// blend = features (the GEMM's A operand) + GEMM; the skinning reads the blend's v_posed
+int launch_blend_features(int n, const float* body_pose, const float* betas, const SmplWorkspace& w, cudaStream_t s);
+int launch_blend_gemm(const SmplDev& m, int n, const SmplWorkspace& w, cudaStream_t s);
+int launch_blend(const SmplDev& m, int n, const float* body_pose, const float* betas, const SmplWorkspace& w, cudaStream_t s);
 int launch_skin(const SmplDev& m, int n, const SmplWorkspace& w, float* vertices, cudaStream_t s);
-int smem_carveout_mask();                    // GLAMR_SMEM_CARVEOUT (see smpl_kernels.cu)
 int lbs_kernel_count(const SmplDev& m);      // kernels one launch_lbs call launches
 int launch_joints_finalize(const SmplDev& m, int n, int orig_joints, const float* root_trans, const float* root_scale,
                            const SmplWorkspace& w, float* joints, cudaStream_t s);

@@ -614,7 +614,7 @@ class GlobalReconOptimizer:
 
     def launches_per_iteration(self):
         """kernels of the CUDA library launched per optimiser iteration for the current stage (excludes the NCCL kernel)"""
-        return int(self._lib.glamr_opt_launch_count(self._opt, int(self.world == 1 or getattr(self, '_peer_ok', False))))
+        return int(self._lib.glamr_opt_launch_count(self._opt))
 
     def _read(self, what, *shape):
         p, n = ctypes.c_void_p(), ctypes.c_size_t()

@@ -224,9 +224,9 @@ int glamr_opt_destroy(glamr_opt_t* st);
 int glamr_opt_set_problem(glamr_opt_t* st, const glamr_problem_t* problem, int reset_adam, void* stream);
 /* length (floats) of the caller-owned reduce buffer: [grad (n_params) | un-normalised term sums (GLAMR_NUM_TERMS)] */
 size_t glamr_opt_reduce_count(const glamr_opt_t* st);
-/* kernels per optimiser iteration for the current problem (bench.py: gpu_launches): via_iterate != 0 for a
- * glamr_opt_iterate loop (Adam fused into the backward tail on one GPU), 0 for a glamr_opt_backward + glamr_opt_apply pair */
-int glamr_opt_launch_count(const glamr_opt_t* st, int via_iterate);
+/* kernels per optimiser iteration for the current problem (bench.py: gpu_launches), the same for a glamr_opt_iterate
+ * loop and for a glamr_opt_backward + glamr_opt_apply pair */
+int glamr_opt_launch_count(const glamr_opt_t* st);
 
 /* forward (trajectory, camera, SMPL, projection) + residuals + analytic backward for the current theta, leaving
  * [grad | term sums] of THIS rank's share in reduce_buf.  With several GPUs the caller sums reduce_buf over ranks

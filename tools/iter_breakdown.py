@@ -18,7 +18,7 @@ m._cur_vars, m._cur_stage, m._loss_cfg = specs['opt_variables'], stage, specs['l
 m._set_stage(data, specs['opt_variables'], specs['loss_cfg'], stage, reset_adam=True, begin=True)
 hist = torch.zeros((400, L.NUM_TERMS + 1), device=dev)
 lib = m._lib
-def it():      # the library's single-GPU iteration (fused head, LBS, fused tail with Adam), eager so that events can sit between launches
+def it():      # the library's single-GPU iteration (forward, LBS, residuals, backward, Adam), eager so that events can sit between launches
     L.check(lib.glamr_opt_iterate(m._opt, L.ptr(m._theta), L.ptr(m._reduce), float(specs['opt_lr']), L.ptr(hist), L.NUM_TERMS + 1, 1, 0, L.stream_ptr()), 'iterate')
 for _ in range(5): it()
 L.check(lib.glamr_opt_kernel_timing(m._opt, 2), 't')

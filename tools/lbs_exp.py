@@ -14,4 +14,4 @@ K = 50
 e0.record()
 for _ in range(K): smpl(global_orient=o, body_pose=p, betas=b, root_trans=t, return_verts=False)
 e1.record(); torch.cuda.synchronize()
-print('N', n, 'stages', os.environ.get('GLAMR_LBS_STAGES'), 'dbg', os.environ.get('GLAMR_LBS_DEBUG'), 'us per smpl forward', e0.elapsed_time(e1)/K*1000)
+print('N', n, 'dbg', os.environ.get('GLAMR_LBS_DEBUG'), 'us per smpl forward', e0.elapsed_time(e1)/K*1000)

@@ -1,5 +1,5 @@
 """Small end-to-end case for compute-sanitizer (memcheck / racecheck): SMPL forward at a ragged size through both LBS paths,
-one prior inference, and a short optimisation through the fused and the legacy iteration kernels.
+one prior inference, and a short optimisation through the iteration kernels.
 
     compute-sanitizer --tool memcheck  python tools/sanitize_case.py
     compute-sanitizer --tool racecheck python tools/sanitize_case.py
