@@ -206,6 +206,19 @@ GLAMR_HD void mat34_mul(const float* A, const float* B, float* o) {
     }
   }
 }
+// person2cam of frame s, corrected by the person's residual variables when it has them:
+// person2cam @ make_transform(person2cam_res_rot, person2cam_res_trans, '6d')  (:484-488).  Returns the 3x4 to use
+// (the constant table itself, or `buf`).
+GLAMR_HD const float* person2cam_at(const OptCtx& c, const glamr_person_t& ps, int s, float* buf) {
+  const float* P2C = ps.person2cam + (size_t)s * 12;
+  if (ps.off_person2cam_res < 0) return P2C;
+  const float* tr = c.theta + ps.off_person2cam_res + 6 * c.pb.T + 3 * s;
+  float R[9];
+  rot6d_to_rotmat(c.theta + ps.off_person2cam_res + 6 * s, R);
+  const float B[12] = {R[0], R[1], R[2], tr[0], R[3], R[4], R[5], tr[1], R[6], R[7], R[8], tr[2]};
+  mat34_mul(P2C, B, buf);
+  return buf;
+}
 // mean over visible persons of person_transform_world @ person2cam at source frame s  (:482-492)
 GLAMR_HD void mean_cam_inv(const OptCtx& c, int s, float* M) {
 #pragma unroll
@@ -213,9 +226,9 @@ GLAMR_HD void mean_cam_inv(const OptCtx& c, int s, float* M) {
   for (int p = 0; p < c.pb.P; ++p) {
     const glamr_person_t& ps = c.pb.persons[p];
     if (ps.vis[s] == 0.0f) continue;
-    float Tw[12], C[12];
+    float Tw[12], C[12], P2C[12];
     person_world_transform(c, p, s, Tw);
-    mat34_mul(Tw, ps.person2cam + (size_t)s * 12, C);
+    mat34_mul(Tw, person2cam_at(c, ps, s, P2C), C);
 #pragma unroll
     for (int k = 0; k < 12; ++k) M[k] += C[k];
   }
@@ -803,7 +816,7 @@ GLAMR_HD void camera_backward(const OptCtx& c, int t, TermAcc& acc) {
   }
 }
 // mode 3 only, after camera_backward of all frames: frame s gathers dL/d(mean) of every frame filled from it and
-// pushes it into dL/d(person_transform_world) of its visible persons.
+// pushes it into dL/d(person_transform_world) of its visible persons (and into their person2cam residuals, if any).
 GLAMR_HD void camera_scatter_to_persons(const OptCtx& c, int s) {
   const glamr_problem_t& pb = c.pb;
   const int T = pb.T;
@@ -822,8 +835,8 @@ GLAMR_HD void camera_scatter_to_persons(const OptCtx& c, int s) {
     const glamr_person_t& ps = pb.persons[p];
     if (ps.vis[s] == 0.0f) continue;
     // M = Tw @ P2C: R_M = Rw Rp, t_M = Rw tp + tw  ->  dRw = G_R Rp^T + G_t tp^T, dtw = G_t
-    const float* P2C = ps.person2cam + (size_t)s * 12;
-    float Rp[9], gRw[9], g[3];
+    float P2Cbuf[12], Rp[9], gRw[9], g[3];
+    const float* P2C = person2cam_at(c, ps, s, P2Cbuf);
     mat34_R(P2C, Rp);
     mat3_mult(G, Rp, gRw);
     const float tp[3] = {P2C[3], P2C[7], P2C[11]};
@@ -835,6 +848,22 @@ GLAMR_HD void camera_scatter_to_persons(const OptCtx& c, int s) {
     aa_to_rotmat_vjp(c.sc.orient_world + n * 3, gRw, g);
 #pragma unroll
     for (int k = 0; k < 3; ++k) { c.sc.g_orient[n * 3 + k] += g[k]; c.sc.g_trans[n * 3 + k] += G[9 + k]; }
+    const int o = ps.off_person2cam_res;
+    if (o >= 0) {
+      // P2C = P2C0 @ [Rr | tr]: R_M = Rw R0 Rr, t_M = Rw (R0 tr + t0) + tw  ->  dRr = (Rw R0)^T G_R, dtr = (Rw R0)^T G_t.
+      // Linear in G like the lines above: with several ranks each writes its share and the all-reduce adds them.
+      float Rw[9], R0[9], A[9], gRr[9], g6[6], gtr[3];
+      aa_to_rotmat(c.sc.orient_world + n * 3, Rw);
+      mat34_R(ps.person2cam + (size_t)s * 12, R0);
+      mat3_mul(Rw, R0, A);
+      mat3_tmul(A, G, gRr);
+      mat3_tvec(A, G + 9, gtr);
+      rot6d_to_rotmat_vjp(c.theta + o + 6 * s, gRr, g6);
+#pragma unroll
+      for (int k = 0; k < 6; ++k) c.sc.grad[o + 6 * s + k] = g6[k];
+#pragma unroll
+      for (int k = 0; k < 3; ++k) c.sc.grad[o + 6 * T + 3 * s + k] = gtr[k];
+    }
   }
 }
 

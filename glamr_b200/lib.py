@@ -44,7 +44,7 @@ _vp = ctypes.c_void_p
 class Person(ctypes.Structure):
     _fields_ = [(n, ctypes.c_int32) for n in
                 ['start', 'len', 'off_xy', 'off_heading', 'off_dxy', 'off_dheading', 'off_z', 'off_rot',
-                 'off_world_dheading', 'off_orient_res', 'off_trans_res', 'pad_']] + \
+                 'off_world_dheading', 'off_orient_res', 'off_trans_res', 'off_person2cam_res']] + \
                [(n, _vp) for n in
                 ['traj_local_pred', 'orient_base_init', 'trans_base_init', 'cam_K', 'kp_target', 'orient_cam_6d',
                  'orient_cam_q', 'trans_cam', 'person2cam', 'dheading_mask', 'rot_mask', 'vis', 'kp_w', 'kp_dist_mask', 'ctr_w', 'ctt_w']]

@@ -19,7 +19,9 @@ from . import lib as L
 
 
 class VariableLayout:
-    def __init__(self, T, n_empty, trans_res_rows, lens):
+    def __init__(self, T, n_empty, trans_res_rows, lens, person2cam_res=False):
+        """person2cam_res: also allocate person2cam_res_rot [T,6] + person2cam_res_trans [T,3] per person
+        (flag_opt_person2cam_rot / _trans), after every other block so that the offsets above do not depend on it"""
         self.T, self.n_empty, self.trans_res_rows, self.lens = T, n_empty, trans_res_rows, list(lens)
         off = 0
 
@@ -35,6 +37,10 @@ class VariableLayout:
         for Ln in self.lens:
             self.persons.append(dict(xy=take(2), heading=take(1), dxy=take(2 * (Ln - 1)), dheading=take(Ln - 1), z=take(Ln),
                                      rot=take(6 * Ln), world_dheading=take(T), orient_res=take(3 * T), trans_res=take(3 * T)))
+        self.person2cam_res = person2cam_res
+        if person2cam_res:
+            for o in self.persons:          # the trans block directly follows the rot block (glamr_person_t.off_person2cam_res)
+                o['p2c_rot'], o['p2c_trans'] = take(6 * T), take(3 * T)
         self.n_params = off
 
     def views(self, theta, p=None):
@@ -48,11 +54,14 @@ class VariableLayout:
                     'cam_inv_trans_residual': v(self.cam_inv_trans_res, 3 * self.trans_res_rows, self.trans_res_rows, 3)}
         o, Ln = self.persons[p], self.lens[p]
         v = lambda k, n, *shape: theta[o[k]:o[k] + n].view(*shape)
-        return {'traj_local_xy': v('xy', 2, 2), 'traj_local_heading': v('heading', 1, 1),
-                'traj_local_dxy': v('dxy', 2 * (Ln - 1), Ln - 1, 2), 'traj_local_dheading': v('dheading', Ln - 1, Ln - 1),
-                'traj_local_z': v('z', Ln, Ln), 'traj_local_rot': v('rot', 6 * Ln, Ln, 6),
-                'world_dheading': v('world_dheading', T, T, 1), 'smpl_orient_world_res': v('orient_res', 3 * T, T, 3),
-                'root_trans_world_res': v('trans_res', 3 * T, T, 3)}
+        out = {'traj_local_xy': v('xy', 2, 2), 'traj_local_heading': v('heading', 1, 1),
+               'traj_local_dxy': v('dxy', 2 * (Ln - 1), Ln - 1, 2), 'traj_local_dheading': v('dheading', Ln - 1, Ln - 1),
+               'traj_local_z': v('z', Ln, Ln), 'traj_local_rot': v('rot', 6 * Ln, Ln, 6),
+               'world_dheading': v('world_dheading', T, T, 1), 'smpl_orient_world_res': v('orient_res', 3 * T, T, 3),
+               'root_trans_world_res': v('trans_res', 3 * T, T, 3)}
+        if self.person2cam_res:
+            out['person2cam_res_rot'], out['person2cam_res_trans'] = v('p2c_rot', 6 * T, T, 6), v('p2c_trans', 3 * T, T, 3)
+        return out
 
 
 def _f32(x, device):
@@ -64,7 +73,8 @@ class StageCompiler:
 
     def __init__(self, data, layout, flags, device, aa_to_rot6d, num_joints=26, aa_to_quat=None):
         """flags: dict with flag_fixed_cam, flag_opt_cam, flag_opt_cam_from_person_pose, flag_cam_inv_trans_res_all,
-        flag_opt_vis_local_rot, cam_fix_frames.  aa_to_rot6d: callable (device math lives in the CUDA library)."""
+        flag_opt_vis_local_rot, cam_fix_frames and optionally flag_opt_person2cam_rot / flag_opt_person2cam_trans (default
+        off).  aa_to_rot6d: callable (device math lives in the CUDA library)."""
         self.data, self.layout, self.flags, self.device, self.J = data, layout, flags, device, num_joints
         self.pids = list(data['person_data'].keys())
         self.P, self.T = len(self.pids), data['seq_len']
@@ -183,6 +193,11 @@ class StageCompiler:
         data, lay, fl, dev, P, T, J = self.data, self.layout, self.flags, self.device, self.P, self.T, self.J
         n_end = P * T if n_end is None else n_end
         for name in loss_cfg:
+            if name == 'person2cam_res_trans_reg':
+                raise NotImplementedError(
+                    "residual 'person2cam_res_trans_reg' fails in the reference itself (loss_func.py:244-245 looks up "
+                    "'person2cam_res_trans' in the top-level data dict, but the variable lives in each person's dict: KeyError), "
+                    "so it has no semantics to match")
             if name not in L.TERM_INDEX:
                 raise NotImplementedError(f"residual '{name}' has no CUDA implementation (no CPU fallback)")
         pb = L.Problem()
@@ -230,6 +245,9 @@ class StageCompiler:
             ps.off_xy, ps.off_heading, ps.off_dxy, ps.off_dheading = o['xy'], o['heading'], o['dxy'], o['dheading']
             ps.off_z, ps.off_rot, ps.off_world_dheading = o['z'], o['rot'], o['world_dheading']
             ps.off_orient_res, ps.off_trans_res = o['orient_res'], o['trans_res']
+            # composed whenever the variables exist (camera-from-persons mode only; a stage that does not optimise them
+            # uses their current value)
+            ps.off_person2cam_res = o['p2c_rot'] if lay.person2cam_res else -1
             for name in ['traj_local_pred', 'orient_base_init', 'trans_base_init', 'cam_K', 'kp_target', 'orient_cam_6d',
                          'orient_cam_q', 'trans_cam', 'person2cam', 'dheading_mask', 'rot_mask', 'vis']:
                 setattr(ps, name, None if c[name] is None else c[name].data_ptr())
@@ -322,7 +340,12 @@ class StageCompiler:
                     on(o[name], sz[name])
                 if key == 'world_dheading':
                     on(o['world_dheading'], T)
-                if key in ('world_dxy', 'person2cam_rot', 'person2cam_trans'):
+                # listed without its flag, the reference does not optimise it (global_recon_model.py:616-619)
+                if key == 'person2cam_rot' and fl.get('flag_opt_person2cam_rot', False):
+                    on(o['p2c_rot'], 6 * T)
+                if key == 'person2cam_trans' and fl.get('flag_opt_person2cam_trans', False):
+                    on(o['p2c_trans'], 3 * T)
+                if key == 'world_dxy':
                     raise NotImplementedError(f"optimisation variable '{key}' is not implemented in the CUDA path")
         active = active.to(dev)
         keep.append(active)
@@ -337,7 +360,8 @@ def make_layout(data, flags):
     T = data['seq_len']
     n_empty = int((torch.as_tensor(data['fr_num_persons']) == 0).sum())
     rows = T if flags['flag_cam_inv_trans_res_all'] else n_empty
-    return VariableLayout(T, n_empty, rows, [int(d['exist_len']) for d in persons.values()])
+    p2c = flags.get('flag_opt_person2cam_rot', False) or flags.get('flag_opt_person2cam_trans', False)
+    return VariableLayout(T, n_empty, rows, [int(d['exist_len']) for d in persons.values()], person2cam_res=p2c)
 
 
 def bind_variables(data, layout, theta):
@@ -349,11 +373,17 @@ def bind_variables(data, layout, theta):
         data[name] = gv[name]
     for p, d in enumerate(data['person_data'].values()):
         pv = layout.views(theta, p)
+        if layout.person2cam_res:
+            # a dict without them (continue_opt from a run without the flags) starts from the initial value of
+            # global_recon_model.py:173-175: identity 6d rotation, zero translation
+            d.setdefault('person2cam_res_rot', torch.tensor([1., 0., 0., 0., 1., 0.]).repeat(layout.T, 1))
+            d.setdefault('person2cam_res_trans', torch.zeros(layout.T, 3))
         for name in ['traj_local_xy', 'traj_local_heading', 'traj_local_dxy', 'traj_local_dheading', 'traj_local_z',
-                     'traj_local_rot', 'smpl_orient_world_res', 'root_trans_world_res', 'world_dheading']:
+                     'traj_local_rot', 'smpl_orient_world_res', 'root_trans_world_res', 'world_dheading',
+                     'person2cam_res_rot', 'person2cam_res_trans']:
             # world_dheading exists once a stage has requested it (global_recon_model.py:624-627); with continue_opt it
             # arrives already optimised and forward() keeps composing with it (:459-465)
-            if name in d:
+            if name in d and name in pv:
                 pv[name].copy_(torch.as_tensor(d[name]).to(theta))
                 d[name] = pv[name]
 

@@ -180,6 +180,8 @@ class GlobalReconOptimizer:
         self.flag_opt_cam = g('flag_opt_cam', True)
         self.flag_fixed_cam = g('flag_fixed_cam', False)
         self.flag_opt_vis_local_rot = g('flag_opt_vis_local_rot', False)
+        self.flag_opt_person2cam_rot = g('flag_opt_person2cam_rot', False)
+        self.flag_opt_person2cam_trans = g('flag_opt_person2cam_trans', False)
         self.flag_cam_inv_trans_res_all = g('flag_cam_inv_trans_res_all', True)
         self.flag_filter_pose = g('flag_filter_pose', True)
         self.flag_make_invis_with_keypoint = g('flag_make_invis_with_keypoint', False)
@@ -189,8 +191,7 @@ class GlobalReconOptimizer:
         self.flag_init_cam_all_frames = g('flag_init_cam_all_frames', False)
         self.cam_fix_frames = g('cam_fix_frames', [[0, None]])
         self.opt_stage_specs = self.cfg.opt_stage_specs
-        for flag in ['flag_opt_motion_latent', 'flag_opt_traj_latent', 'flag_use_pen_loss', 'flag_traj_from_cam', 'absolute_heading',
-                     'flag_opt_person2cam_rot', 'flag_opt_person2cam_trans']:
+        for flag in ['flag_opt_motion_latent', 'flag_opt_traj_latent', 'flag_use_pen_loss', 'flag_traj_from_cam', 'absolute_heading']:
             if g(flag, False):
                 raise NotImplementedError(f'{flag} is not implemented in the CUDA path (SURVEY.md §8(f)-4); no CPU fallback')
         if g('heading_type', 'scalar') != 'scalar':
@@ -216,7 +217,8 @@ class GlobalReconOptimizer:
     @property
     def _flags(self):
         return {k: getattr(self, k) for k in ['flag_fixed_cam', 'flag_opt_cam', 'flag_opt_cam_from_person_pose',
-                                              'flag_cam_inv_trans_res_all', 'flag_opt_vis_local_rot', 'cam_fix_frames']}
+                                              'flag_cam_inv_trans_res_all', 'flag_opt_vis_local_rot', 'cam_fix_frames',
+                                              'flag_opt_person2cam_rot', 'flag_opt_person2cam_trans']}
 
     # ------------------------------------------------------------------------------------------------ init_data
     def _person_from_estimate(self, est, gt_entry):
@@ -456,6 +458,9 @@ class GlobalReconOptimizer:
             d['person2cam'] = G.inverse_transform(d['person_transform_cam'])
         last = d
         for d in persons.values():
+            if self.flag_opt_person2cam_rot or self.flag_opt_person2cam_trans:         # :173-175, all T frames
+                d['person2cam_res_rot'] = torch.tensor([1., 0., 0., 0., 1., 0.], device=dev).repeat(num_fr, 1)
+                d['person2cam_res_trans'] = torch.zeros(num_fr, 3, device=dev)
             d['smpl_orient_world_res'] = torch.zeros_like(last['smpl_orient_world'])
             d['root_trans_world_res'] = torch.zeros_like(last['root_trans_world'])
         rel = {}

@@ -156,7 +156,9 @@ typedef struct glamr_person {
   int32_t start, len;              /* exist range [start, start+len) of this person (exist_frames)              */
   int32_t off_xy, off_heading, off_dxy, off_dheading, off_z, off_rot;     /* offsets into theta (floats)        */
   int32_t off_world_dheading, off_orient_res, off_trans_res;              /* [T], [T,3], [T,3]                  */
-  int32_t pad_;
+  int32_t off_person2cam_res;      /* person2cam_res_rot [T,6] followed directly by person2cam_res_trans [T,3], or -1
+                                    * (flag_opt_person2cam_* off).  GLAMR_CAM_FROM_PERSONS composes
+                                    * person2cam @ [R(rot6d) | trans] (global_recon_model.py:484-488)           */
   const float* traj_local_pred;    /* [len,11]                                                                    */
   const float* orient_base_init;   /* [T,3] smpl_orient_world_base outside the exist range                        */
   const float* trans_base_init;    /* [T,3]                                                                       */
@@ -165,7 +167,7 @@ typedef struct glamr_person {
   const float* orient_cam_6d;      /* [T,6]  rot6d(R(smpl_orient_cam)), target of cam_traj_rot                    */
   const float* orient_cam_q;       /* [T,4]  angle_axis_to_quaternion(smpl_orient_cam): target when rot_type 'quat' */
   const float* trans_cam;          /* [T,3]  root_trans_cam                                                       */
-  const float* person2cam;         /* [T,12] 3x4, used by GLAMR_CAM_FROM_PERSONS                                  */
+  const float* person2cam;         /* [T,12] 3x4, used by GLAMR_CAM_FROM_PERSONS (before the residual above)      */
   const float* dheading_mask;      /* [len-1] (cam_fix_frames)                                                    */
   const float* rot_mask;           /* [len] or NULL (flag_opt_vis_local_rot)                                      */
   const float* vis;                /* [T] 1/0 vis_frames                                                          */
